@@ -220,10 +220,46 @@ def unit_plan(total_images: int, world: int, B: int, sub: int):
     return plan
 
 
+def dump_records(out_dir: str, records) -> None:
+    """Score records [n, 14] of one step -> out_dir/<field>.npy (float32), the fields DetectionPipeline.detect_device
+    returns (risk_probs as [n, 5]).  The bench's weights and images are seeded, so two builds can be compared field by field."""
+    import numpy as np
+
+    from dfd import pipeline
+
+    os.makedirs(out_dir, exist_ok=True)
+    rec = records.float().cpu().numpy()
+    fields = pipeline.PACKED_FIELDS
+    n_scalar = fields.index("risk_p0")
+    for i, name in enumerate(fields[:n_scalar]):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(rec[:, i]))
+    np.save(os.path.join(out_dir, "risk_probs.npy"), np.ascontiguousarray(rec[:, n_scalar:]))
+
+
+def seeded_workload(arch, B: int, local: int, max_batch: int, fuse_ln: bool = True, precise_residual: bool = False,
+                    graphs: bool = True):
+    """The pipeline the bench times (seeded random weights of `arch`) and its B seeded u8 images on cuda:local.  Every rank
+    draws the same images: the records of a work-queue unit do not depend on which rank took it."""
+    import torch
+
+    from dfd import pipeline, scoring, weights
+
+    dev = torch.device("cuda", local)
+    bsd = weights.random_vision_state_dict(arch, seed=0, device=dev)
+    st = scoring.ScoringStack(dev, weights.random_freq_mlp_g2(2), weights.random_fusion_g2(3), [-1.0, -0.2, 0.3, 1.5], 1.0)
+    pipe = pipeline.DetectionPipeline(arch, bsd, weights.random_classifier_head("B", arch.hidden_size, 1), st, device=local,
+                                      max_batch=max_batch, fuse_ln=fuse_ln, precise_residual=precise_residual, graphs=graphs)
+    del bsd
+    S = arch.image_size
+    g = torch.Generator(device=dev).manual_seed(1234)
+    images = torch.randint(0, 256, (B, S, S, 3), dtype=torch.uint8, device=dev, generator=g)
+    return pipe, images
+
+
 def run_ours(args):
     import torch
 
-    from dfd import _lib, distributed, pipeline, scoring, weights
+    from dfd import _lib, distributed, pipeline
     from dfd.engine import ARCHS
 
     if not torch.cuda.is_available():
@@ -246,15 +282,9 @@ def run_ours(args):
     sub = args.sub_batch or (B if (world == 1 or strong) else max(1, B // 2))
     sub = min(sub, B)
 
-    bsd = weights.random_vision_state_dict(arch, seed=0, device=dev)
-    st = scoring.ScoringStack(dev, weights.random_freq_mlp_g2(2), weights.random_fusion_g2(3), [-1.0, -0.2, 0.3, 1.5], 1.0)
-    pipe = pipeline.DetectionPipeline(arch, bsd, weights.random_classifier_head("B", arch.hidden_size, 1), st,
-                                      device=local, max_batch=min(sub, args.max_batch), fuse_ln=bool(args.fuse_ln),
-                                      precise_residual=bool(args.precise_residual), graphs=bool(args.graphs))
-    del bsd
+    pipe, images = seeded_workload(arch, B, local, max_batch=min(sub, args.max_batch), fuse_ln=bool(args.fuse_ln),
+                                   precise_residual=bool(args.precise_residual), graphs=bool(args.graphs))
     S = arch.image_size
-    g = torch.Generator(device=dev).manual_seed(1234 + rank)
-    images = torch.randint(0, 256, (B, S, S, 3), dtype=torch.uint8, device=dev, generator=g)
     F = len(pipeline.PACKED_FIELDS)
 
     def unit_images(unit, src):
@@ -331,6 +361,8 @@ def run_ours(args):
     replays = pipe.engine.graph_replays - replays0
     clocks = sampler.stop()
     value = world * B * args.steps / dt
+    if args.dump_outputs and rank == 0:      # after gather(): the slab holds every rank's records
+        dump_records(args.dump_outputs, slab[(args.steps - 1) * per_step:])
 
     # ---- profiled pass (not part of `value`): the same work with every launch of the engine bracketed by CUDA events on its
     # stream (eager launches), read back once at the end — per-family / per-GEMM-type durations for the roofline entries
@@ -525,7 +557,7 @@ def run_latency(args):
             for mode in ("eager", "graph"):
                 pipe.engine.set_graphs(mode == "graph")
                 r0 = pipe.engine.graph_replays
-                ms = _event_ms(lambda: pipe.pack(pipe.detect_device(x, None, clahe=True)), iters=max(args.steps, 20))
+                ms = _event_ms(lambda: pipe.pack(pipe.detect_device(x, None, clahe=True)), iters=args.steps)
                 row[mode + "_ms"] = ms
                 if mode == "graph":
                     row["graph_replays"] = pipe.engine.graph_replays - r0
@@ -535,7 +567,7 @@ def run_latency(args):
         del pipe
     print(json.dumps({"metric": "detection step latency, small batches (u8 images resident in HBM -> score records on the device)",
                       "unit": "ms", "value": out["so400m-384/B=6"]["graph_ms"], "higher_is_better": False, "n_gpus": 1,
-                      "steps": max(args.steps, 20), "warmup": 3, "dtype": "bf16", "data": "synthetic",
+                      "steps": args.steps, "warmup": 3, "dtype": "bf16", "data": "synthetic",
                       "config": {"workload": "latency: 1 / 6 / 9 / 32 views per call, base-224 and so400m-384, eager vs CUDA graph"},
                       "gpu_launches": int(_lib.load().dfd_launch_count()), "table": out}), flush=True)
 
@@ -553,12 +585,12 @@ def run_cifake(args):
     name = WORKLOADS["base-224"][0]
     model = dropin.FastBinaryClassifier("small", device=dev, arch=name, max_batch=1024,
                                         head_state=weights.random_fast_classifier_head("small", ARCHS[name].hidden_size))
-    sweep = cifake.throughput_sweep(model, batches=(256, 512, 1024, 2048, 4096, 8192), side=32, iters=max(args.steps, 3))
+    sweep = cifake.throughput_sweep(model, batches=(256, 512, 1024, 2048, 4096, 8192), side=32, iters=args.steps)
     best = max(sweep, key=sweep.get)
     arch = model.arch
     peaks = load_peaks()
     print(json.dumps({"metric": "images/sec CiFake 32->224 binary classifier (FastBinaryClassifier, base-patch16-224)",
-                      "unit": "images/s", "value": sweep[best], "higher_is_better": True, "n_gpus": 1, "steps": max(args.steps, 3),
+                      "unit": "images/s", "value": sweep[best], "higher_is_better": True, "n_gpus": 1, "steps": args.steps,
                       "warmup": 1, "dtype": "bf16", "data": "synthetic",
                       "config": {"workload": "cifake: 32x32 u8 -> bilinear 224 in the patch kernel -> backbone -> head H-D",
                                  "best_batch": best, "engine_max_batch": 1024},
@@ -589,7 +621,7 @@ def run_head_train(args):
     t0 = time.perf_counter()
     train_fusion.fit_fusion_head(zf, zs, y, batch_size=32, epochs=1, device=dev, verbose=False)       # warm-up epoch
     torch.cuda.synchronize()
-    epochs = max(args.steps, 3)
+    epochs = args.steps
     t0 = time.perf_counter()
     train_fusion.fit_fusion_head(zf, zs, y, batch_size=32, epochs=epochs, device=dev, verbose=False)
     torch.cuda.synchronize()
@@ -643,7 +675,7 @@ def run_library(args):
             with torch.inference_mode(), torch.autocast("cuda", dtype=torch.bfloat16):
                 return m(pixel_values=x).pooler_output
 
-        ms = _event_ms(step, iters=max(args.steps, 5), warm=max(args.warmup, 3))
+        ms = _event_ms(step, iters=args.steps, warm=max(args.warmup, 3))
         ips = B / ms * 1e3
         table[wl] = {"batch": B, "ms_per_step": ms, "images_per_s": ips,
                      "tensor_pipe_frac_of_sustained": a.flops_per_image() * ips / 1e12 / float(peaks["bf16_tflops_sustained"])}
@@ -651,7 +683,7 @@ def run_library(args):
         torch.cuda.empty_cache()
     print(json.dumps({"metric": "images/sec, backbone only, transformers.SiglipVisionModel eager on one B200 (library comparison point)",
                       "impl": "library", "unit": "images/s", "value": table["so400m-384"]["images_per_s"], "higher_is_better": True,
-                      "n_gpus": 1, "steps": max(args.steps, 5), "warmup": max(args.warmup, 3), "dtype": "bf16 autocast", "data": "synthetic",
+                      "n_gpus": 1, "steps": args.steps, "warmup": max(args.warmup, 3), "dtype": "bf16 autocast", "data": "synthetic",
                       "config": {"workload": "library: HF SiglipVisionModel, bf16 autocast + SDPA, inference_mode, fp32 NCHW input on the device; "
                                              "so400m-384 and base-224"},
                       "gpu_launches": 0, "table": table}), flush=True)
@@ -660,7 +692,8 @@ def run_library(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 5; latency 20 calls per shape, cifake 3 calls per batch, head-train 3 epochs)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--workload", choices=sorted(WORKLOADS) + ["latency", "cifake", "head-train", "library"], default="so400m-384",
@@ -680,7 +713,15 @@ def main():
                     help="1 = two-bf16 residual stream (dfd_engine_set_precise_residual): the reference's fp32 residual "
                          "accumulation, a few percent slower; 0 = the default bf16 stream")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the score records of the last timed step to DIR/<field>.npy (float32), to compare two builds")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = {"latency": 20, "cifake": 3, "head-train": 3}.get(args.workload, 5)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs covers the so400m-384 and base-224 workloads of --impl ours")
     if args.impl == "reference":
         if args.workload not in WORKLOADS:
             raise SystemExit("--impl reference covers the so400m-384 and base-224 workloads")

@@ -4,19 +4,24 @@ checkpoint's `backbone.*` tensors into it through their own load paths (inferenc
 train_fusion_head_only.py:111-124).  No forward runs here (no GPU: the tower is a parameter skeleton and its forward
 raises); the numerics of the same flow are checked on the GPU in tests/test_dropin_gpu.py.
 
-/root/reference only exists in the build container; the tests that read it skip elsewhere.
+The reference's source is not part of this repository: the tests that exec it read a checkout named by DFD_REFERENCE_DIR
+and skip without one.  They also pin tests/reference_style.py, the restatement of the same classes that the test_restated_*
+tests here and the GPU tests drive on every machine, to the originals (same parameters, same loaded tensors).
 """
 import ast
 import os
 import sys
 import types
+import warnings
 
 import pytest
 import torch
 import torch.nn as nn
 
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources are not present on this box")
+from tests.reference_style import load_siglip_from_best, reference_style_classifier
+
+REF = os.environ.get("DFD_REFERENCE_DIR", "")
+needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="DFD_REFERENCE_DIR does not name a checkout of the reference")
 
 
 def _extract(path, names):
@@ -59,15 +64,19 @@ def _checkpoint_like(model, seed):
     return ck
 
 
-@needs_ref
-def test_reference_inference_classifier_strict_load_reaches_the_backbone(shims):
-    """inference_ai_human_images.py: `BinaryClassifier(nn.Module)` + its strict load (:841-846)."""
-    import open_clip  # the stand-in
+def _param_shapes(model):
+    return {k: tuple(v.shape) for k, v in model.state_dict().items()}
 
-    ns = {"torch": torch, "nn": nn, "open_clip": open_clip, "print": lambda *a, **k: None}
-    exec(_extract(os.path.join(REF, "inference_ai_human_images.py"), ["BinaryClassifier"]), ns)
+
+def _restated(kind, shims):
+    name, img_size = ("ViT-B-16-SigLIP-384", 64) if kind == "A" else ("ViT-L-16-SigLIP-384", 60)
+    return reference_style_classifier(kind, name, shims.ARCHS[name].hidden_size, img_size)
+
+
+def _check_inference_classifier_strict_load(make):
+    """The load path of inference_ai_human_images.py (:841-857) on the model `make()` builds; returns the model."""
     with pytest.warns(UserWarning, match="random"):   # pretrained='webli' cannot be fetched: said loudly, not silently
-        model = ns["BinaryClassifier"](model_size="small", device="cpu").to("cpu")
+        model = make()
     assert isinstance(model.backbone, nn.Module) and "backbone" in dict(model.named_children())
     names = [k for k, _ in model.named_parameters()]
     assert "backbone.visual.trunk.blocks.1.attn.qkv.weight" in names            # timm names (simple_classifier.py:491)
@@ -85,26 +94,42 @@ def test_reference_inference_classifier_strict_load_reaches_the_backbone(shims):
     assert model.backbone.weights_source == "checkpoint"
     with pytest.raises(RuntimeError, match="CUDA"):
         model(torch.zeros(1, 3, 64, 64))       # no CPU fallback: the forward fails loudly
+    return model
 
 
 @needs_ref
-def test_reference_fusion_trainer_loader_reaches_the_backbone(shims, tmp_path):
-    """train_fusion_head_only.py: `BinaryClassifier`, `_filter_state_for_model`, `load_siglip_from_best` (:78-124)."""
-    import open_clip
-    from safetensors.torch import load_file, save_file
+def test_reference_inference_classifier_strict_load_reaches_the_backbone(shims):
+    """inference_ai_human_images.py: `BinaryClassifier(nn.Module)` + its strict load (:841-846)."""
+    import open_clip  # the stand-in
 
-    D = shims.ARCHS["ViT-L-16-SigLIP-384"].hidden_size
-    ns = {"torch": torch, "nn": nn, "open_clip": open_clip, "load_file": load_file, "SIGLIP_DIM": D, "IMG_SIZE": 60,
-          "DEVICE": "cpu", "print": lambda *a, **k: None}
-    exec(_extract(os.path.join(REF, "train_fusion_head_only.py"),
-                  ["BinaryClassifier", "_filter_state_for_model", "load_siglip_from_best"]), ns)
+    ns = {"torch": torch, "nn": nn, "open_clip": open_clip, "print": lambda *a, **k: None}
+    exec(_extract(os.path.join(REF, "inference_ai_human_images.py"), ["BinaryClassifier"]), ns)
+    model = _check_inference_classifier_strict_load(lambda: ns["BinaryClassifier"](model_size="small", device="cpu").to("cpu"))
+    # the restatement the other tests drive declares the same submodules and parameters
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        restated = _restated("A", shims)("cpu")
+    assert [n for n, _ in restated.named_children()] == [n for n, _ in model.named_children()]
+    assert _param_shapes(restated) == _param_shapes(model)
+
+
+def test_restated_inference_classifier_strict_load_reaches_the_backbone(shims):
+    """The same load path on tests/reference_style.py's restatement of that class (no reference checkout needed)."""
+    _check_inference_classifier_strict_load(lambda: _restated("A", shims)("cpu").to("cpu"))
+
+
+def _check_fusion_trainer_loader(classifier, load_from_best, tmp_path):
+    """`load_siglip_from_best` of train_fusion_head_only.py (:111-124) on a synthetic `best_model` checkpoint of `classifier`:
+    every trunk tensor arrives.  Returns (probe, loaded model, checkpoint path)."""
+    from safetensors.torch import save_file
+
     with pytest.warns(UserWarning):
-        probe = ns["BinaryClassifier"]("cpu")
+        probe = classifier("cpu")
     ck = _checkpoint_like(probe, 2)
     path = os.path.join(tmp_path, "best_model.safetensors")
     save_file({k: v.contiguous() for k, v in ck.items()}, path)
     with pytest.warns(UserWarning):
-        model = ns["load_siglip_from_best"](path)
+        model = load_from_best(path)
     assert model.backbone.weights_source == "checkpoint"
     sd = model.state_dict()
     n_backbone = 0
@@ -112,6 +137,36 @@ def test_reference_fusion_trainer_loader_reaches_the_backbone(shims, tmp_path):
         assert torch.equal(v, ck[k]), k
         n_backbone += k.startswith("backbone.visual.trunk.")
     assert n_backbone == 12 * probe.backbone.arch.num_hidden_layers + 18   # every trunk tensor went through the filter
+    return probe, model, path
+
+
+@needs_ref
+def test_reference_fusion_trainer_loader_reaches_the_backbone(shims, tmp_path):
+    """train_fusion_head_only.py: `BinaryClassifier`, `_filter_state_for_model`, `load_siglip_from_best` (:78-124)."""
+    import open_clip
+    from safetensors.torch import load_file
+
+    D = shims.ARCHS["ViT-L-16-SigLIP-384"].hidden_size
+    ns = {"torch": torch, "nn": nn, "open_clip": open_clip, "load_file": load_file, "SIGLIP_DIM": D, "IMG_SIZE": 60,
+          "DEVICE": "cpu", "print": lambda *a, **k: None}
+    exec(_extract(os.path.join(REF, "train_fusion_head_only.py"),
+                  ["BinaryClassifier", "_filter_state_for_model", "load_siglip_from_best"]), ns)
+    probe, model, path = _check_fusion_trainer_loader(ns["BinaryClassifier"], ns["load_siglip_from_best"], tmp_path)
+    # the restatement declares the same submodules and parameters, and its loader delivers the same tensors
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        restated = _restated("B", shims)
+        assert [n for n, _ in restated("cpu").named_children()] == [n for n, _ in probe.named_children()]
+        assert _param_shapes(restated("cpu")) == _param_shapes(probe)
+        mine = load_siglip_from_best(restated, path)
+    theirs = model.state_dict()
+    assert all(torch.equal(v, theirs[k]) for k, v in mine.state_dict().items())
+
+
+def test_restated_fusion_trainer_loader_reaches_the_backbone(shims, tmp_path):
+    """The same loader on tests/reference_style.py's restatement (no reference checkout needed)."""
+    restated = _restated("B", shims)
+    _check_fusion_trainer_loader(restated, lambda path: load_siglip_from_best(restated, path), tmp_path)
 
 
 def test_tower_accepts_hf_layout_and_round_trips_timm_names():

@@ -5,6 +5,8 @@ import numpy as np
 import pytest
 import torch
 
+from tests.reference_style import reference_style_classifier
+
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 
@@ -481,47 +483,9 @@ def test_siglip2_mtl_end_to_end():
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# The reference's own flow on the GPU.  /root/reference does not exist on the GPU box, so the two model classes are
-# restated here the way the reference declares them (same submodule names, same forward; the source-extracted originals
-# run against the same shims in tests/test_dropin_cpu.py) and driven like its entry points drive them.
+# The reference's own flow on the GPU, with its two model classes as tests/reference_style.py restates them (checked
+# against the reference's source in tests/test_dropin_cpu.py where a checkout is given), driven like its entry points drive them.
 # ---------------------------------------------------------------------------------------------------------------------
-def _reference_style_classifier(kind, arch_name, dim, img_size):
-    """kind 'A': inference_ai_human_images.py:111-152; kind 'B': train_fusion_head_only.py:78-109."""
-    import open_clip  # the dfd stand-in (install_import_shims)
-    import torch.nn as nn
-
-    class BinaryClassifierA(nn.Module):
-        def __init__(self, device):
-            super().__init__()
-            self.resolution = img_size
-            self.backbone, _, self.preprocess = open_clip.create_model_and_transforms(arch_name, pretrained="webli", device=device)
-            self.classifier = nn.Sequential(nn.LayerNorm(dim), nn.Dropout(0.3), nn.Linear(dim, dim // 2), nn.GELU(),
-                                            nn.Dropout(0.2), nn.Linear(dim // 2, 1))
-
-        def forward(self, x):
-            features = self.backbone.encode_image(x)
-            features = features / features.norm(dim=-1, keepdim=True)
-            return self.classifier(features).squeeze(-1)
-
-    class BinaryClassifierB(nn.Module):
-        def __init__(self, device):
-            super().__init__()
-            self.backbone, _, _ = open_clip.create_model_and_transforms(arch_name, pretrained="webli", device=device)
-            self.se = nn.Sequential(nn.Linear(dim, dim // 16), nn.ReLU(), nn.Linear(dim // 16, dim), nn.Sigmoid())
-            self.classifier = nn.Sequential(nn.LayerNorm(dim), nn.Dropout(0.3), nn.Linear(dim, dim // 2), nn.GELU(),
-                                            nn.Dropout(0.2), nn.Linear(dim // 2, dim // 4), nn.GELU(), nn.Linear(dim // 4, 1))
-
-        def forward(self, x):
-            with torch.no_grad():
-                if x.shape[-1] != img_size:
-                    x = nn.functional.interpolate(x, size=(img_size, img_size))
-                f = self.backbone.encode_image(x)
-                f = f / (f.norm(dim=-1, keepdim=True) + 1e-6)
-            return self.classifier(f * self.se(f)).squeeze(-1)
-
-    return BinaryClassifierA if kind == "A" else BinaryClassifierB
-
-
 def _timm_checkpoint(sd, hs):
     """`best_model` checkpoint as the reference's trainers write it: open_clip/timm backbone names + head + text tower."""
     from dfd import dropin
@@ -551,7 +515,7 @@ def test_reference_style_module_strict_load_inference_mode_autocast(kind, eps):
     sd, hs = R.init_state_dict(c, 0), R.init_head(kind, c.hidden_size, 1)
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        model = _reference_style_classifier(kind, name, c.hidden_size, c.image_size)(DEV).to(DEV)
+        model = reference_style_classifier(kind, name, c.hidden_size, c.image_size)(DEV).to(DEV)
     assert model.backbone.weights_source == "random"
     x = R.preprocess_u8(R.synthetic_images(6, c.image_size, 3))
     model.eval()
@@ -598,7 +562,7 @@ def test_reference_style_module_survives_torch_compile():
     sd, hs = R.init_state_dict(c, 0), R.init_head("A", c.hidden_size, 1)
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        model = _reference_style_classifier("A", name, c.hidden_size, c.image_size)(DEV).to(DEV).eval()
+        model = reference_style_classifier("A", name, c.hidden_size, c.image_size)(DEV).to(DEV).eval()
     model.load_state_dict(_timm_checkpoint(sd, hs), strict=True)
     x = R.preprocess_u8(R.synthetic_images(4, c.image_size, 3)).to(DEV)
     with torch.inference_mode():

@@ -412,3 +412,44 @@ def test_cuda_graph_replay_is_bit_equal_to_eager(fuse_ln):
     assert torch.equal(graph(buf[6])[0], eager(buf[6])[0]) and graph.graph_replays == 9
     eager.close()
     graph.close()
+
+
+def test_bench_dump_outputs_are_the_last_steps_records(tmp_path):
+    """bench.py --dump-outputs: one float32 .npy per field of the last timed step's score records.  Each field equals what
+    DetectionPipeline.detect_device returns for the bench's seeded weights and images (bench.seeded_workload, run here in
+    process), for runs with 1 and 3 timed steps; the JSON line reports the requested number of timed steps."""
+    import importlib.util
+    import json
+    import os
+    import subprocess
+    import sys
+
+    import numpy as np
+
+    from dfd import pipeline
+    from dfd.engine import ARCHS
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    names = list(pipeline.PACKED_FIELDS[:pipeline.PACKED_FIELDS.index("risk_p0")]) + ["risk_probs"]
+    B, arch_name = 16, bench.WORKLOADS["base-224"][0]
+    pipe, images = bench.seeded_workload(ARCHS[arch_name], B, 0, max_batch=B)
+    out = pipe.detect_device(images, None, clahe=True)
+    want = {n: out[n].float().cpu().numpy() for n in names}
+    pipe.engine.close()
+    for steps in (1, 3):
+        d = tmp_path / f"steps{steps}"
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "base-224", "--batch", str(B),
+                            "--steps", str(steps), "--warmup", "0", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=900, cwd=tmp_path)
+        assert r.returncode == 0, r.stderr[-3000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        assert sorted(os.listdir(d)) == sorted(n + ".npy" for n in names)
+        for n in names:
+            got = np.load(d / (n + ".npy"))
+            assert got.dtype == np.float32 and got.shape == want[n].shape, (n, got.dtype, got.shape)
+            # the frequency features sum per-CTA partials with a double-precision atomicAdd: allow last-bit differences
+            assert np.allclose(got, want[n], rtol=1e-5, atol=1e-6), (n, float(np.abs(got - want[n]).max()))
+        assert np.array_equal(np.load(d / "risk_idx.npy"), want["risk_idx"])
