@@ -36,7 +36,6 @@ class GemmEpilogue(C.Structure):
         ("residual_op", C.c_int),
         ("ln_parts", C.c_int),
         ("residual_lo", C.c_void_p),
-        ("ldlo", C.c_int64),
     ]
 
 
@@ -106,9 +105,7 @@ SIGNATURES = {
     "dfd_gemm_last_variant": (_I, []),
     "dfd_gemm_variant_launches": (_L, [_I]),
     "dfd_gemm_bf16_tile": (_I, [_P, _L, _P, _L, _P, _L, _I, _I, _I, C.POINTER(GemmEpilogue), _I, _P]),
-    "dfd_layernorm_bf16": (_I, [_P, _L, _P, _L, _P, _P, _I, _I, _F, _P]),
-    "dfd_layernorm2_bf16": (_I, [_P, _L, _P, _L, _P, _L, _P, _P, _I, _I, _F, _P]),
-    "dfd_rowstats_bf16": (_I, [_P, _L, _P, _I, _I, _P]),
+    "dfd_layernorm_bf16": (_I, [_P, _L, _P, _P, _L, _P, _P, _I, _I, _F, _P]),
     "dfd_attention_bf16": (_I, [_P, _L, _P, _L, _I, _I, _I, _I, _F, _P]),
     "dfd_attention_bf16_impl": (_I, [_P, _L, _P, _L, _I, _I, _I, _I, _F, _I, _P]),
     "dfd_patchify": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _L, _P]),
@@ -116,15 +113,11 @@ SIGNATURES = {
     "dfd_head_fwd": (_I, [C.POINTER(HeadWeights), _P, _L, _I, _P, _P, _P, _P, _P]),
     "dfd_freq_features": (_I, [_P, _I, _P, _F, _I, _P, _P, _P]),
     "dfd_freq_scratch_bytes": (_L, [_I]),
-    "dfd_resample_ksize": (_I, [_I, _I]),
-    "dfd_resample_coeffs_host": (_I, [_I, _I, _P, _P, _P]),
+    "dfd_resample_ksize": (_I, [_I, _I, _I]),
+    "dfd_resample_coeffs_host": (_I, [_I, _I, _I, _P, _P, _P]),
     "dfd_gray256_scratch_bytes": (_L, [_I, _I, _I]),
-    "dfd_resample_ksize_filter": (_I, [_I, _I, _I]),
-    "dfd_resample_coeffs_filter_host": (_I, [_I, _I, _I, _P, _P, _P]),
-    "dfd_resize_u8": (_I, [_P, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _I, _P, _P, _P]),
-    "dfd_gray256": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _I, _P, _P, _P]),
-    "dfd_gray256_strided": (_I, [_P, _L, _L, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _I, _P, _P, _P]),
-    "dfd_resize_u8_strided": (_I, [_P, _L, _L, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _I, _P, _P, _P]),
+    "dfd_resize_u8": (_I, [_P, _L, _L, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _I, _P, _P, _P]),
+    "dfd_gray256": (_I, [_P, _L, _L, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _I, _P, _P, _P]),
     "dfd_clahe_scratch_bytes": (_L, [_I, _I]),
     "dfd_clahe_u8": (_I, [_P, _I, _I, _I, _I, _P, _P, _P]),
     "dfd_score_epilogue": (_I, [C.POINTER(ScoreWeights), _P, _P, _P, _I, C.POINTER(Scores), _P]),
@@ -145,7 +138,6 @@ SIGNATURES = {
     "dfd_engine_graph_replays": (C.c_int64, [_P]),
     "dfd_engine_profile": (_I, [_P, _I]),
     "dfd_engine_profile_read": (_I, [_P, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
-    "dfd_engine_profile_read_families": (_I, [_P, _I, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
 }
 
 _lib = None

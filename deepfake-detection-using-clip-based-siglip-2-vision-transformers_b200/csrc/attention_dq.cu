@@ -41,14 +41,17 @@ constexpr int kThreads = 352;    // loader, 2 MMA warps, 2 x 4 softmax warps
 constexpr int kTmemCols = 512;
 constexpr int kColO = 256;
 constexpr int kColQ = 416;
-// HANDOFF = pairs of exponentials (of 32 per row and tile) a tile issues before it hands the MUFU turn to the other tile: measured on
+// kHandoff = pairs of exponentials (of 32 per row and tile) a tile issues before it hands the MUFU turn to the other tile: measured on
 // B200 at so400m shapes (64 images): 8 -> 0.253 ms, 16 -> 0.247, 24 -> 0.249, 32 (strict alternation) -> 0.277
+constexpr int kHandoff = 16;
 
 // 2^x for a pair on the FMA pipe (x <= ~8): round to the nearest integer with the 1.5·2^23 trick, degree-3 minimax polynomial
 // of 2^f on [-0.5, 0.5] (7.5e-5 relative: P is rounded to bf16, 2e-3, right after), exponent added as an integer.  The MUFU
 // unit takes 8 cycles per warp-wide EX2 and the softmax warps are what bounds this kernel (scripts/ubench_softmax.cu:
 // 10.8 cycles per exponential and scheduler with two warps per scheduler, all on the MUFU unit; 9.0 with every third pair
-// here), so a share of the exponentials goes through six packed FMA-pipe instructions per pair instead.
+// here), so a share of the exponentials goes through six packed FMA-pipe instructions per pair instead: every kPoly-th pair
+// (every 3rd and all on the MUFU unit measured slower, profiles/r02_attention.md §C).
+constexpr int kPoly = 4;
 __device__ __forceinline__ float2 poly_exp2x2(float2 x) {
   const float kMagic = 12582912.0f;
   x.x = fmaxf(x.x, -120.0f);
@@ -113,7 +116,7 @@ __device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, const void* s
                : "memory");
 }
 
-template <int HD, int POLY, int HANDOFF>
+template <int HD>
 __global__ void __launch_bounds__(kThreads, 1)
 attention_dq_kernel(const __grid_constant__ CUtensorMap tmMain, const __grid_constant__ CUtensorMap tmTail,
                     const __grid_constant__ CUtensorMap tmOut, int N, int H, int n_items, float scale_log2) {
@@ -374,7 +377,7 @@ attention_dq_kernel(const __grid_constant__ CUtensorMap tmMain, const __grid_con
     uint32_t su0 = 0, su1 = 0;   // s_full uses per S buffer
     uint32_t g = 0, it = 0;      // running count of this tile's P·V products (o_done phases), item count
     uint32_t act_items = 0;      // items in which this tile was active (o_full phases)
-    if (HANDOFF > 0 && t == 1 && lane == 0) mbar_arrive(&turn[0]);   // tile 0 takes the first turn
+    if (t == 1 && lane == 0) mbar_arrive(&turn[0]);   // tile 0 takes the first turn
     if (blockIdx.x < n_items) copy_q(0);
     for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++it) {
       const int qp = item % QP, h = (item / QP) % H, b = item / (QP * H);
@@ -383,12 +386,10 @@ attention_dq_kernel(const __grid_constant__ CUtensorMap tmMain, const __grid_con
       if (row0 >= N) {  // (only tile 1) nothing to do for this item; keep the turn-taking and the Q hand-shake going
         // (turns first: the next item's Q only arrives after the loader has placed all of THIS item's K/V stages, and
         //  those drain only as tile 0 advances - which needs its turns)
-        if (HANDOFF > 0) {
-          for (int j = 0; j < T; ++j) {
-            mbar_wait(&turn[t], turns++ & 1u);
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&turn[t ^ 1]);
-          }
+        for (int j = 0; j < T; ++j) {
+          mbar_wait(&turn[t], turns++ & 1u);
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&turn[t ^ 1]);
         }
         if (has_next) copy_q(it + 1);
         continue;
@@ -444,35 +445,32 @@ attention_dq_kernel(const __grid_constant__ CUtensorMap tmMain, const __grid_con
         m = m_new;
         float2 sum4[4] = {{0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}};
         const float2 sc2 = make_float2(scale_log2, scale_log2), nm2 = make_float2(-m, -m);
-        if (HANDOFF > 0) mbar_wait(&turn[t], turns++ & 1u);      // ---- this tile's turn on the MUFU unit ----
-        // packed FFMA2 / FADD2 around the exponentials; every POLY-th pair is computed on the FMA pipe instead
+        mbar_wait(&turn[t], turns++ & 1u);      // ---- this tile's turn on the MUFU unit ----
+        // packed FFMA2 / FADD2 around the exponentials; every kPoly-th pair is computed on the FMA pipe instead
         auto exps = [&](int c) {
           const float2 x = ffma2(make_float2(__uint_as_float(s[2 * c]), __uint_as_float(s[2 * c + 1])), sc2, nm2);
           float2 p;
-          if (POLY > 0 && (c % (POLY > 0 ? POLY : 1)) == POLY - 1) p = poly_exp2x2(x);
+          if (c % kPoly == kPoly - 1) p = poly_exp2x2(x);
           else p = make_float2(fast_exp2(x.x), fast_exp2(x.y));
           sum4[c & 3] = fadd2(sum4[c & 3], p);
           s[c] = pack_bf16x2(p.x, p.y);  // in place: s[2c], s[2c+1] (indices >= c) are consumed first
         };
-        constexpr int kFirst = HANDOFF > 0 ? HANDOFF : 16;   // pairs before the hand-off (and before the short-tile cut)
 #pragma unroll
-        for (int c = 0; c < kFirst; ++c) exps(c);
-        if (HANDOFF > 0) {
-          // ---- hand the MUFU unit to the other tile after kHandoff of the 32 pairs: its first exponentials then fill the
-          // gaps of this warp's last ones (one warp cannot saturate the unit).  The arrive is predicated on a partial row sum
-          // (never negative; ptxas cannot know): a data dependence on the exponentials before it, otherwise the predicated
-          // arrive is scheduled ahead of most of them
-          const float2 pa = fadd2(fadd2(sum4[0], sum4[1]), fadd2(sum4[2], sum4[3]));
-          __syncwarp();
-          if (lane == 0 && pa.x + pa.y >= 0.f) mbar_arrive(&turn[t ^ 1]);
-        }
-        if (valid > 2 * kFirst) {
+        for (int c = 0; c < kHandoff; ++c) exps(c);
+        // ---- hand the MUFU unit to the other tile after kHandoff of the 32 pairs: its first exponentials then fill the
+        // gaps of this warp's last ones (one warp cannot saturate the unit).  The arrive is predicated on a partial row sum
+        // (never negative; ptxas cannot know): a data dependence on the exponentials before it, otherwise the predicated
+        // arrive is scheduled ahead of most of them
+        const float2 pa = fadd2(fadd2(sum4[0], sum4[1]), fadd2(sum4[2], sum4[3]));
+        __syncwarp();
+        if (lane == 0 && pa.x + pa.y >= 0.f) mbar_arrive(&turn[t ^ 1]);
+        if (valid > 2 * kHandoff) {
 #pragma unroll
-          for (int c = kFirst; c < 32; ++c) exps(c);
+          for (int c = kHandoff; c < 32; ++c) exps(c);
         } else {
           // short last tile (so400m: 25 of 64 keys): the rest of the row is all padding, P = 0 without exponentials
 #pragma unroll
-          for (int c = kFirst; c < 32; ++c) s[c] = 0u;
+          for (int c = kHandoff; c < 32; ++c) s[c] = 0u;
         }
         const float2 sa = fadd2(fadd2(sum4[0], sum4[1]), fadd2(sum4[2], sum4[3]));
         const float lsum = sa.x + sa.y;
@@ -581,10 +579,8 @@ int make_tmap_qkv_4d(CUtensorMap* out, const void* base, int hd, int heads3, int
                          swizzle32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_128B, false);
 }
 
-// variant = 100 * poly + handoff: every poly-th pair of exponentials runs on the FMA pipe (0 = all on the MUFU unit); a tile
-// hands the MUFU turn over after `handoff` of its 32 pairs (0 = no turns)
 int attention_dq_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, int B, int N, int H, int hd,
-                      float scale, cudaStream_t st, int variant) {
+                      float scale, cudaStream_t st) {
   DFD_REQUIRE(qkv && out, DFD_ERR_BAD_ARG, "attention: null pointer");
   DFD_REQUIRE(B > 0 && N > 0 && H > 0, DFD_ERR_SHAPE, "attention: B, N, H must be positive");
   DFD_REQUIRE(hd == 64 || hd == 72, DFD_ERR_UNSUPPORTED, "attention: head dim %d not supported (64, 72)", hd);
@@ -608,29 +604,14 @@ int attention_dq_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, in
   const float scale_log2 = scale * 1.4426950408889634f;
   const int n_items = (int)items64;
   const int grid = n_items < kNumSMs ? n_items : kNumSMs;
-  static SmemOptIn smem_once[2][3];
-#define DFD_DQ_LAUNCH(HD_, POLY_, HO_, SLOT_)                                                                              \
+  static SmemOptIn smem_once[2];
+#define DFD_DQ_LAUNCH(HD_)                                                                                                  \
   do {                                                                                                                      \
-    if (int rc2 = ensure_dynamic_smem(smem_once[HD_ == 64 ? 0 : 1][SLOT_], attention_dq_kernel<HD_, POLY_, HO_>,            \
-                                      DqSmem<HD_>::kTotal))                                                                 \
+    if (int rc2 = ensure_dynamic_smem(smem_once[HD_ == 64 ? 0 : 1], attention_dq_kernel<HD_>, DqSmem<HD_>::kTotal))         \
       return rc2;                                                                                                           \
-    attention_dq_kernel<HD_, POLY_, HO_><<<grid, kThreads, DqSmem<HD_>::kTotal, st>>>(tmMain, tmTail, tmOut, N, H, n_items, \
-                                                                                     scale_log2);                          \
+    attention_dq_kernel<HD_><<<grid, kThreads, DqSmem<HD_>::kTotal, st>>>(tmMain, tmTail, tmOut, N, H, n_items, scale_log2); \
   } while (0)
-  // variant = 100 * poly + handoff.  The product is kDqVariantDefault (every 4th pair of exponentials on the FMA pipe, turn
-  // hand-over after 16 pairs); 16 (all exponentials on the MUFU unit) and 316 stay as A/B hooks.  Hand-over after 8 / 24 pairs,
-  // no turns, and every 2nd pair were measured and dropped (profiles/r02_attention.md §C).
-#define DFD_DQ_VARIANTS(HD_)                                         \
-  switch (variant) {                                                 \
-    case 16: DFD_DQ_LAUNCH(HD_, 0, 16, 0); break;                    \
-    case 316: DFD_DQ_LAUNCH(HD_, 3, 16, 1); break;                   \
-    case 416: DFD_DQ_LAUNCH(HD_, 4, 16, 2); break;                   \
-    default:                                                         \
-      set_last_error("attention: unknown dq variant %d", variant);   \
-      return DFD_ERR_BAD_ARG;                                        \
-  }
-  if (hd == 64) { DFD_DQ_VARIANTS(64) } else { DFD_DQ_VARIANTS(72) }
-#undef DFD_DQ_VARIANTS
+  if (hd == 64) DFD_DQ_LAUNCH(64); else DFD_DQ_LAUNCH(72);
 #undef DFD_DQ_LAUNCH
   DFD_LAUNCH_CHECK();
   g_launches.fetch_add(1, std::memory_order_relaxed);
@@ -647,7 +628,7 @@ namespace dfd {
 int attention_auto_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, int B, int N, int H, int hd,
                         float scale, cudaStream_t st) {
   if (N <= 128) return attention_ws_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st);
-  return attention_dq_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st, kDqVariantDefault);
+  return attention_dq_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st);
 }
 
 }  // namespace dfd
@@ -663,9 +644,7 @@ extern "C" DFD_API int dfd_attention_bf16_impl(const void* qkv, int64_t ldqkv, v
                                                int H, int hd, float scale, int impl, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (impl == 2) return dfd::attention_ws_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st);
-  if (impl == 5) return dfd::attention_dq_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st, 16);
-  if (impl == 6) return dfd::attention_dq_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st, 316);
-  if (impl == 7) return dfd::attention_dq_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st, 416);
-  dfd::set_last_error("attention: impl must be 2 (single-tile persistent) or 5 / 6 / 7 (dual-query-tile: exponentials all on the MUFU unit / every 3rd / every 4th pair on the FMA pipe)");
+  if (impl == 5) return dfd::attention_dq_bf16(qkv, ldqkv, out, ldo, B, N, H, hd, scale, st);
+  dfd::set_last_error("attention: impl must be 2 (single-tile persistent) or 5 (dual-query-tile)");
   return DFD_ERR_BAD_ARG;
 }

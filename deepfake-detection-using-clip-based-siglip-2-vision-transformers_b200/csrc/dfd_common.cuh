@@ -71,16 +71,12 @@ inline int ensure_dynamic_smem(SmemOptIn& once, F func, int bytes) {
 // ---------------------------------------------------------------------------------------------
 int gemm_bf16_dispatch(const void* A, int64_t lda, const void* W, int64_t ldw, void* C, int64_t ldc,
                        int M, int N, int K, const dfd_gemm_epilogue* epi, int force_bn, cudaStream_t st);
-int layernorm_bf16(const void* x, int64_t ldx, void* y, int64_t ldy, const float* gamma,
-                   const float* beta, int M, int D, float eps, cudaStream_t st, const void* lo = nullptr,
-                   int64_t ldlo = 0);
-int rowstats_bf16(const void* x, int64_t ldx, float* stats, int M, int D, cudaStream_t st);
+int layernorm_bf16(const void* x, int64_t ldx, const void* lo, void* y, int64_t ldy, const float* gamma,
+                   const float* beta, int M, int D, float eps, cudaStream_t st);
 int patchify(const void* pixels, int pix_format, int B, int Hin, int Win, int S, int P, int resize_mode,
              void* A, int64_t lda, cudaStream_t st);
-// attention_dq variant = 100 * poly + handoff (see attention_dq.cu)
-constexpr int kDqVariantDefault = 416;
 int attention_dq_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, int B, int N, int H, int hd,
-                      float scale, cudaStream_t st, int variant = kDqVariantDefault);
+                      float scale, cudaStream_t st);
 int attention_auto_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, int B, int N, int H, int hd,
                         float scale, cudaStream_t st);
 int attention_ws_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, int B, int N, int H, int hd,

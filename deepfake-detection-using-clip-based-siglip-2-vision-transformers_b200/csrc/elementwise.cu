@@ -1,8 +1,7 @@
-// HBM-bound row kernels of the backbone: LayerNorm, row statistics, fused preprocess + im2col.
+// HBM-bound row kernels of the backbone: LayerNorm, fused preprocess + im2col.
 //
 //   dfd_layernorm_bf16  one warp per token row, 16-byte loads, fp32 two-pass statistics
 //                       (HF:modeling_siglip.py:348,357,618 — nn.LayerNorm(eps=1e-6) under autocast runs in fp32)
-//   dfd_rowstats_bf16   (Σx, Σx²) per row for the LN-folded GEMM epilogue
 //   dfd_patchify        u8 NHWC / f32 NCHW pixels → normalised bf16 patch matrix, optional nearest /
 //                       bilinear resample (inference_ai_human_images.py:200-204; train_fusion_head_only.py:67-74,103-104;
 //                       cifake_binary_classifier.py:716-717; HF:modeling_siglip.py:124-130,178)
@@ -36,7 +35,7 @@ __device__ __forceinline__ float2 ln_val(const uint4& hi, const uint4& lo, int j
 // LO: the row is the sum of two bf16 tensors (x + lo: the two-bf16 residual stream of the precise engine mode)
 template <bool LO>
 __global__ void __launch_bounds__(kRowThreads)
-layernorm_bf16_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, const __nv_bfloat16* __restrict__ lo, int64_t ldlo,
+layernorm_bf16_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, const __nv_bfloat16* __restrict__ lo,
                       __nv_bfloat16* __restrict__ y, int64_t ldy, const float* __restrict__ gamma,
                       const float* __restrict__ beta, int M, int D, float eps) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -94,33 +93,6 @@ layernorm_bf16_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, const __
       o.w = pack_bf16x2((d.x - mean) * rstd * g1.z + b1.z, (d.y - mean) * rstd * g1.w + b1.w);
       yr[c] = o;
     }
-  }
-}
-
-__global__ void __launch_bounds__(kRowThreads)
-rowstats_bf16_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, float* __restrict__ stats, int M,
-                     int D) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int row = blockIdx.x * (kRowThreads / 32) + warp;
-  if (row >= M) return;
-  const int nvec = D >> 3;
-  const uint4* xr = reinterpret_cast<const uint4*>(x + (int64_t)row * ldx);
-  float s = 0.f, q = 0.f;
-  for (int c = lane; c < nvec; c += 32) {
-    const uint4 v = __ldg(xr + c);
-    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float2 a = unpack_bf16x2(w[j]);
-      s += a.x + a.y;
-      q += a.x * a.x + a.y * a.y;
-    }
-  }
-  s = warp_sum(s);
-  q = warp_sum(q);
-  if (lane == 0) {
-    stats[2 * (int64_t)row] = s;
-    stats[2 * (int64_t)row + 1] = q;
   }
 }
 
@@ -261,37 +233,24 @@ __global__ void __launch_bounds__(256) patchify_u8_rows_kernel(PatchArgs a) {
 
 }  // namespace
 
-int layernorm_bf16(const void* x, int64_t ldx, void* y, int64_t ldy, const float* gamma,
-                   const float* beta, int M, int D, float eps, cudaStream_t st, const void* lo, int64_t ldlo) {
+int layernorm_bf16(const void* x, int64_t ldx, const void* lo, void* y, int64_t ldy, const float* gamma,
+                   const float* beta, int M, int D, float eps, cudaStream_t st) {
   DFD_REQUIRE(x && y && gamma && beta, DFD_ERR_BAD_ARG, "layernorm: null pointer");
   DFD_REQUIRE(M > 0 && D > 0, DFD_ERR_SHAPE, "layernorm: M and D must be positive");
   DFD_REQUIRE(D % 8 == 0 && D <= kMaxVec * 256, DFD_ERR_SHAPE,
               "layernorm: D must be a multiple of 8 and <= %d (D=%d)", kMaxVec * 256, D);
   DFD_REQUIRE(ldx % 8 == 0 && ldy % 8 == 0 && ldx >= D && ldy >= D, DFD_ERR_SHAPE,
               "layernorm: leading dimensions must be multiples of 8 and >= D");
-  (void)ldlo;   // the low halves are tiled: their layout is a function of D
   const int rows_per_cta = kRowThreads / 32;
   const int grid = (M + rows_per_cta - 1) / rows_per_cta;
   if (lo != nullptr)
     layernorm_bf16_kernel<true><<<grid, kRowThreads, 0, st>>>(
-        reinterpret_cast<const __nv_bfloat16*>(x), ldx, reinterpret_cast<const __nv_bfloat16*>(lo), ldlo,
+        reinterpret_cast<const __nv_bfloat16*>(x), ldx, reinterpret_cast<const __nv_bfloat16*>(lo),
         reinterpret_cast<__nv_bfloat16*>(y), ldy, gamma, beta, M, D, eps);
   else
     layernorm_bf16_kernel<false><<<grid, kRowThreads, 0, st>>>(
-        reinterpret_cast<const __nv_bfloat16*>(x), ldx, nullptr, 0, reinterpret_cast<__nv_bfloat16*>(y), ldy, gamma,
-        beta, M, D, eps);
-  DFD_LAUNCH_CHECK();
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  return DFD_OK;
-}
-
-int rowstats_bf16(const void* x, int64_t ldx, float* stats, int M, int D, cudaStream_t st) {
-  DFD_REQUIRE(x && stats, DFD_ERR_BAD_ARG, "rowstats: null pointer");
-  DFD_REQUIRE(M > 0 && D > 0 && D % 8 == 0 && ldx % 8 == 0 && ldx >= D, DFD_ERR_SHAPE,
-              "rowstats: bad shape (M=%d D=%d ldx=%lld)", M, D, (long long)ldx);
-  const int rows_per_cta = kRowThreads / 32;
-  rowstats_bf16_kernel<<<(M + rows_per_cta - 1) / rows_per_cta, kRowThreads, 0, st>>>(
-      reinterpret_cast<const __nv_bfloat16*>(x), ldx, stats, M, D);
+        reinterpret_cast<const __nv_bfloat16*>(x), ldx, nullptr, reinterpret_cast<__nv_bfloat16*>(y), ldy, gamma, beta,
+        M, D, eps);
   DFD_LAUNCH_CHECK();
   g_launches.fetch_add(1, std::memory_order_relaxed);
   return DFD_OK;
@@ -346,22 +305,9 @@ int patchify(const void* pixels, int pix_format, int B, int Hin, int Win, int S,
 
 }  // namespace dfd
 
-// LayerNorm of the two-bf16 row x + lo (the residual stream of dfd_engine_set_precise_residual)
-extern "C" DFD_API int dfd_layernorm2_bf16(const void* x, int64_t ldx, const void* lo, int64_t ldlo, void* y, int64_t ldy,
-                                           const float* gamma, const float* beta, int M, int D, float eps, void* stream) {
-  DFD_REQUIRE(lo != nullptr, DFD_ERR_BAD_ARG, "layernorm2: null pointer");
-  return dfd::layernorm_bf16(x, ldx, y, ldy, gamma, beta, M, D, eps, reinterpret_cast<cudaStream_t>(stream), lo, ldlo);
-}
-
-extern "C" DFD_API int dfd_layernorm_bf16(const void* x, int64_t ldx, void* y, int64_t ldy,
-                                          const float* gamma, const float* beta, int M, int D,
-                                          float eps, void* stream) {
-  return dfd::layernorm_bf16(x, ldx, y, ldy, gamma, beta, M, D, eps,
-                             reinterpret_cast<cudaStream_t>(stream));
-}
-extern "C" DFD_API int dfd_rowstats_bf16(const void* x, int64_t ldx, float* stats, int M, int D,
-                                         void* stream) {
-  return dfd::rowstats_bf16(x, ldx, stats, M, D, reinterpret_cast<cudaStream_t>(stream));
+extern "C" DFD_API int dfd_layernorm_bf16(const void* x, int64_t ldx, const void* lo, void* y, int64_t ldy,
+                                          const float* gamma, const float* beta, int M, int D, float eps, void* stream) {
+  return dfd::layernorm_bf16(x, ldx, lo, y, ldy, gamma, beta, M, D, eps, reinterpret_cast<cudaStream_t>(stream));
 }
 extern "C" DFD_API int dfd_patchify(const void* pixels, int pix_format, int B, int Hin, int Win, int S,
                                     int P, int resize_mode, void* A, int64_t lda, void* stream) {

@@ -516,30 +516,22 @@ extern "C" DFD_API int dfd_engine_profile(dfd_engine* e, int enable) {
 // Sums the event-timed durations of every launch recorded since the last read (or since profiling was switched on) per
 // kernel family (ms) and the launch counts, then clears the record.  Synchronises on the last recorded event.
 // Families: 0 GEMM (patch embedding, pooling head), 1 attention, 2 LayerNorm, 3 patchify, 4 MAP attention, 5 qkv GEMM,
-// 6 out-projection GEMM, 7 fc1 GEMM, 8 fc2 GEMM.  With n <= 5 the encoder GEMMs (5..8) count as family 0 and families >= n
-// fold into n - 1 (the four- and five-family forms of earlier callers).
-extern "C" DFD_API int dfd_engine_profile_read_families(dfd_engine* e, int n, float* ms, int* count) {
-  DFD_REQUIRE(e && ms && count && n > 0, DFD_ERR_BAD_ARG, "profile_read: null pointer");
+// 6 out-projection GEMM, 7 fc1 GEMM, 8 fc2 GEMM.
+extern "C" DFD_API int dfd_engine_profile_read(dfd_engine* e, float* ms, int* count) {
+  DFD_REQUIRE(e && ms && count, DFD_ERR_BAD_ARG, "profile_read: null pointer");
   DeviceGuard guard(e->device);
-  for (int i = 0; i < n; ++i) { ms[i] = 0.f; count[i] = 0; }
+  for (int i = 0; i < 9; ++i) { ms[i] = 0.f; count[i] = 0; }
   if (e->prof_n == 0) return DFD_OK;
   DFD_CUDA(cudaEventSynchronize(e->prof_ev[2 * e->prof_n - 1]));
   for (int i = 0; i < e->prof_n; ++i) {
     float t = 0.f;
     DFD_CUDA(cudaEventElapsedTime(&t, e->prof_ev[2 * i], e->prof_ev[2 * i + 1]));
-    int f = e->prof_fam[i];
-    if (n <= 5 && f >= 5) f = 0;
-    if (f >= n) f = n - 1;
+    const int f = e->prof_fam[i];
     ms[f] += t;
     count[f] += 1;
   }
   e->prof_n = 0;
   return DFD_OK;
-}
-
-// the four-family form of round 1: GEMM, attention, LayerNorm, other (patchify + MAP attention)
-extern "C" DFD_API int dfd_engine_profile_read(dfd_engine* e, float* ms4, int* count4) {
-  return dfd_engine_profile_read_families(e, 4, ms4, count4);
 }
 
 // The launches of one forward, enqueued on st (which may be a capturing stream).
@@ -580,7 +572,7 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
       ep.ln_eps = eps;
       DFD_OP(5, gemm_bf16_dispatch(e->x, D, l.w_qkv, D, e->qkv, 3 * D, M, 3 * D, D, &ep, 0, st));
     } else {
-      DFD_OP(2, layernorm_bf16(e->x, D, e->h, D, l.ln1_g, l.ln1_b, M, D, eps, st, lo, D));
+      DFD_OP(2, layernorm_bf16(e->x, D, lo, e->h, D, l.ln1_g, l.ln1_b, M, D, eps, st));
       dfd_gemm_epilogue ep{};
       ep.bias = l.b_qkv;
       DFD_OP(5, gemm_bf16_dispatch(e->h, D, l.w_qkv, D, e->qkv, 3 * D, M, 3 * D, D, &ep, 0, st));
@@ -592,7 +584,6 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
       ep.residual = e->x;
       ep.ldr = D;
       ep.residual_lo = lo;
-      ep.ldlo = D;
       if (fuse) ep.stats_out = e->stats_b;
       DFD_OP(6, gemm_bf16_dispatch(e->att, D, l.w_o, D, e->x, D, M, D, D, &ep, 0, st));
     }
@@ -607,7 +598,7 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
       ep.ln_eps = eps;
       DFD_OP(7, gemm_bf16_dispatch(e->x, D, l.w_fc1, D, e->mlp, I, M, I, D, &ep, 0, st));
     } else {
-      DFD_OP(2, layernorm_bf16(e->x, D, e->h, D, l.ln2_g, l.ln2_b, M, D, eps, st, lo, D));
+      DFD_OP(2, layernorm_bf16(e->x, D, lo, e->h, D, l.ln2_g, l.ln2_b, M, D, eps, st));
       dfd_gemm_epilogue ep{};
       ep.bias = l.b_fc1;
       ep.act = 1;
@@ -619,7 +610,6 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
       ep.residual = e->x;
       ep.ldr = D;
       ep.residual_lo = lo;
-      ep.ldlo = D;
       if (fuse && li + 1 < e->L) ep.stats_out = e->stats_a;  // for the next layer's LN1 (the post-LN runs as a kernel)
       DFD_OP(8, gemm_bf16_dispatch(e->mlp, I, l.w_fc2, I, e->x, D, M, D, I, &ep, 0, st));
     }
@@ -628,7 +618,7 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
                                cudaMemcpyDeviceToDevice, st));
   }
   __nv_bfloat16* xp = last_hidden ? reinterpret_cast<__nv_bfloat16*>(last_hidden) : e->h;
-  DFD_OP(2, layernorm_bf16(e->x, D, xp, D, e->post_g, e->post_b, M, D, eps, st, lo, D));
+  DFD_OP(2, layernorm_bf16(e->x, D, lo, xp, D, e->post_g, e->post_b, M, D, eps, st));
   {  // K | V projection of every token (rows D..3D of in_proj)
     dfd_gemm_epilogue ep{};
     ep.bias = e->b_in + D;
@@ -640,7 +630,7 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
     ep.bias = e->b_mo;
     DFD_OP(0, gemm_bf16_dispatch(e->ao, D, e->w_mo, D, e->r, D, B, D, D, &ep, 0, st));
   }
-  DFD_OP(2, layernorm_bf16(e->r, D, e->h2, D, e->hln_g, e->hln_b, B, D, eps, st));
+  DFD_OP(2, layernorm_bf16(e->r, D, nullptr, e->h2, D, e->hln_g, e->hln_b, B, D, eps, st));
   {
     dfd_gemm_epilogue ep{};
     ep.bias = e->b_mfc1;

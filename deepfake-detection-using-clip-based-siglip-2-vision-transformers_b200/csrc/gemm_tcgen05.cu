@@ -48,7 +48,6 @@ struct EpiArgs {
   int ln_parts;     // ln_rowstats holds this many partial (Σx, Σx²) pairs per row: [ln_parts][M][2]
   __nv_bfloat16* lo;  // low half of a two-bf16 ("hi + lo") residual stream, tiled (see the epilogue): read with the residual,
                       // written with C
-  int64_t ldlo;       // unused (the tiled layout is a function of N)
 };
 
 // CG = CTAs per MMA (1, or 2 = cta_group::2: a 256 x BN tile shared by an SM pair, each CTA staging its own
@@ -699,7 +698,6 @@ int gemm_bf16_dispatch(const void* A, int64_t lda, const void* W, int64_t ldw, v
     ea.residual_op = epi->residual_op;
     ea.ln_parts = epi->ln_parts > 0 ? epi->ln_parts : 1;
     ea.lo = reinterpret_cast<__nv_bfloat16*>(epi->residual_lo);
-    ea.ldlo = epi->ldlo;
     DFD_REQUIRE(ea.lo == nullptr || (uintptr_t)ea.lo % 16 == 0, DFD_ERR_SHAPE, "gemm: residual_lo must be 16-byte aligned");
     DFD_REQUIRE(ea.lo == nullptr || ea.residual_op == 0, DFD_ERR_BAD_ARG, "gemm: residual_lo goes with an additive residual");
     DFD_REQUIRE(ea.act >= 0 && ea.act <= 3, DFD_ERR_BAD_ARG, "gemm: act must be 0 (none), 1 (gelu_tanh), 2 (gelu_erf) or 3 (sigmoid)");

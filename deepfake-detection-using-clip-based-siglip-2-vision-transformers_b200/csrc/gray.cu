@@ -10,8 +10,8 @@
 //   luma_kernel              RGB u8 NHWC -> L u8                         (Pillow Convert.c rgb2l)
 //   clahe_lut_kernel         per (image, tile): histogram in shared memory, clip + redistribute, prefix sum -> LUT
 //   clahe_apply_kernel       per pixel: bilinear blend of the 4 surrounding tile LUTs        (OpenCV clahe.cpp)
-//   resample_rows_kernel     horizontal pass, u8 -> u8                    (Pillow Resample.c, 8bpc)
-//   resample_cols_kernel     vertical pass, u8 -> f32 / 255
+//   resize_rows_kernel       horizontal pass, u8 -> u8                    (Pillow Resample.c, 8bpc)
+//   resize_cols_kernel       vertical pass, u8 -> f32 / 255
 // HBM-bound streaming kernels; ~1.3 MB of traffic per 384x384 image, < 0.1 % of the detection step.
 #include "dfd_common.cuh"
 
@@ -74,6 +74,28 @@ __device__ __forceinline__ int reflect101(int i, int n) {
   if (n == 1) return 0;
   while (i < 0 || i >= n) i = i < 0 ? -i : 2 * (n - 1) - i;
   return i;
+}
+
+// OpenCV's tile geometry for an H x W plane: tile size (the image extended to a multiple of 8 when 8 does not divide it),
+// histogram clip limit (clipLimit 2.0 scaled to the tile area, at least 1) and the LUT scale 255 / area
+struct ClaheGeometry {
+  int tw, th, clip;
+  float lut_scale;
+};
+ClaheGeometry clahe_geometry(int H, int W) {
+  ClaheGeometry g;
+  if (W % kTiles == 0 && H % kTiles == 0) {
+    g.tw = W / kTiles;
+    g.th = H / kTiles;
+  } else {
+    g.tw = (W + (kTiles - W % kTiles)) / kTiles;
+    g.th = (H + (kTiles - H % kTiles)) / kTiles;
+  }
+  const int area = g.tw * g.th;
+  g.lut_scale = 255.0f / (float)area;
+  g.clip = (int)(2.0 * area / 256);
+  if (g.clip < 1) g.clip = 1;
+  return g;
 }
 
 // grid (64 tiles, B·C planes), 256 threads.  tile (tw x th) of the image extended by BORDER_REFLECT_101 to a multiple of 8.
@@ -292,36 +314,9 @@ clahe_apply_band_kernel(const uint8_t* __restrict__ L, const uint8_t* __restrict
 // ---------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int clip8(int acc) { return min(max(acc >> kPrecisionBits, 0), 255); }
 
-// in [B, H, W] u8 -> out [B, H, 256] u8 ; one thread per output pixel, a block covers one row
-__global__ void __launch_bounds__(kOut)
-resample_rows_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, int H, int W,
-                     const int* __restrict__ xmin, const int* __restrict__ count, const int* __restrict__ kk,
-                     int ksize) {
-  const int xx = threadIdx.x, y = blockIdx.x, b = blockIdx.y;
-  const uint8_t* row = in + ((int64_t)b * H + y) * W;
-  const int x0 = xmin[xx], n = count[xx];
-  const int* k = kk + xx * ksize;
-  int acc = 1 << (kPrecisionBits - 1);
-  for (int i = 0; i < n; ++i) acc += (int)row[x0 + i] * __ldg(k + i);
-  out[((int64_t)b * H + y) * kOut + xx] = (uint8_t)clip8(acc);
-}
-
-// in [B, H, 256] u8 -> out [B, 256, 256] f32 = u8 / 255 ; a block covers one output row
-__global__ void __launch_bounds__(kOut)
-resample_cols_kernel(const uint8_t* __restrict__ in, float* __restrict__ out, int H, const int* __restrict__ ymin,
-                     const int* __restrict__ count, const int* __restrict__ kk, int ksize) {
-  const int x = threadIdx.x, yy = blockIdx.x, b = blockIdx.y;
-  const uint8_t* img = in + (int64_t)b * H * kOut;
-  const int y0 = ymin[yy], n = count[yy];
-  const int* k = kk + yy * ksize;
-  int acc = 1 << (kPrecisionBits - 1);
-  for (int i = 0; i < n; ++i) acc += (int)img[(int64_t)(y0 + i) * kOut + x] * __ldg(k + i);
-  out[((int64_t)b * kOut + yy) * kOut + x] = __fdiv_rn((float)clip8(acc), 255.0f);
-}
-
 // Fast forms of the two passes for tables with at most kTapMax taps (384 -> 256: 7, 224 -> 256: 5).  Rows pass: a thread owns
 // one output column, keeps that column's window and coefficients in registers and walks kRowsPerCta image rows staged in shared
-// memory by word loads (the generic kernel re-reads the table for every output pixel and runs one tiny CTA per row).  Columns
+// memory by word loads (the generic kernel re-reads the table for every output pixel and runs one CTA per row).  Columns
 // pass: a thread produces 4 adjacent pixels of 4 output rows from 32-bit loads and writes float4s.
 constexpr int kTapMax = 8;
 constexpr int kRowsPerCta = 16;
@@ -385,7 +380,8 @@ resample_cols_fast_kernel(const uint8_t* __restrict__ in, float* __restrict__ ou
   }
 }
 
-// Generic Pillow 8bpc passes for interleaved images (C = 1 or 3 channels): used by dfd_resize_u8
+// Generic Pillow 8bpc passes for interleaved images (C = 1 or 3 channels): dfd_resize_u8, and gray256 where the fast forms do
+// not apply (C = 1, OW = OH = 256, f32 output)
 // in [B, H, W, C] -> out [B, H, OW, C]
 __global__ void __launch_bounds__(256)
 resize_rows_kernel(const uint8_t* __restrict__ in, int64_t row_stride, int64_t image_stride, uint8_t* __restrict__ out, int H,
@@ -402,9 +398,12 @@ resize_rows_kernel(const uint8_t* __restrict__ in, int64_t row_stride, int64_t i
   for (int i = 0; i < n; ++i) acc += (int)row[(x0 + i) * C] * __ldg(k + i);
   out[((int64_t)b * H + y) * OW * C + e] = (uint8_t)clip8(acc);
 }
-// in [B, H, OW, C] -> out [B, OH, OW, C]
+__device__ __forceinline__ void store_px(uint8_t* p, int v) { *p = (uint8_t)v; }
+__device__ __forceinline__ void store_px(float* p, int v) { *p = __fdiv_rn((float)v, 255.0f); }
+// in [B, H, OW, C] -> out [B, OH, OW, C], u8 or f32 = u8 / 255
+template <typename T>
 __global__ void __launch_bounds__(256)
-resize_cols_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, int H, int OH, int OWC,
+resize_cols_kernel(const uint8_t* __restrict__ in, T* __restrict__ out, int H, int OH, int OWC,
                    const int* __restrict__ ymin, const int* __restrict__ count, const int* __restrict__ kk, int ksize) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   const int yy = blockIdx.y, b = blockIdx.z;
@@ -414,7 +413,7 @@ resize_cols_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, in
   const int* k = kk + yy * ksize;
   int acc = 1 << (kPrecisionBits - 1);
   for (int i = 0; i < n; ++i) acc += (int)img[(int64_t)(y0 + i) * OWC] * __ldg(k + i);
-  out[((int64_t)b * OH + yy) * OWC + e] = (uint8_t)clip8(acc);
+  store_px(out + ((int64_t)b * OH + yy) * OWC + e, clip8(acc));
 }
 
 double bilinear_filter(double x) {
@@ -433,7 +432,7 @@ double bicubic_filter(double x) {
 }  // namespace
 
 // filter: DFD_FILTER_BILINEAR (support 1) or DFD_FILTER_BICUBIC (support 2)
-int resample_ksize(int in_size, int out_size, int filter = DFD_FILTER_BICUBIC) {
+int resample_ksize(int in_size, int out_size, int filter) {
   double filterscale = (double)in_size / out_size;
   if (filterscale < 1.0) filterscale = 1.0;
   const double support = (filter == DFD_FILTER_BILINEAR ? 1.0 : 2.0) * filterscale;
@@ -442,25 +441,15 @@ int resample_ksize(int in_size, int out_size, int filter = DFD_FILTER_BICUBIC) {
 
 }  // namespace dfd
 
-// Pillow precompute_coeffs + normalize_coeffs_8bpc for the bicubic filter over the whole axis (host, double
-// precision, the library's operation order).  kk must hold out_size * dfd_resample_ksize(in, out) ints.
-extern "C" DFD_API int dfd_resample_ksize(int in_size, int out_size) {
-  if (in_size <= 0 || out_size <= 0) return 0;
-  return dfd::resample_ksize(in_size, out_size);
-}
-
-extern "C" DFD_API int dfd_resample_ksize_filter(int in_size, int out_size, int filter) {
+extern "C" DFD_API int dfd_resample_ksize(int in_size, int out_size, int filter) {
   if (in_size <= 0 || out_size <= 0 || (filter != DFD_FILTER_BILINEAR && filter != DFD_FILTER_BICUBIC)) return 0;
   return dfd::resample_ksize(in_size, out_size, filter);
 }
 
-extern "C" DFD_API int dfd_resample_coeffs_host(int in_size, int out_size, int32_t* xmin_host, int32_t* count_host,
-                                                int32_t* kk_host) {
-  return dfd_resample_coeffs_filter_host(in_size, out_size, DFD_FILTER_BICUBIC, xmin_host, count_host, kk_host);
-}
-
-extern "C" DFD_API int dfd_resample_coeffs_filter_host(int in_size, int out_size, int filter, int32_t* xmin_host,
-                                                       int32_t* count_host, int32_t* kk_host) {
+// Pillow precompute_coeffs + normalize_coeffs_8bpc over the whole axis (host, double precision, the library's operation
+// order).  kk must hold out_size * dfd_resample_ksize(in, out, filter) ints.
+extern "C" DFD_API int dfd_resample_coeffs_host(int in_size, int out_size, int filter, int32_t* xmin_host,
+                                                int32_t* count_host, int32_t* kk_host) {
   DFD_REQUIRE(in_size > 0 && out_size > 0 && xmin_host && count_host && kk_host, DFD_ERR_BAD_ARG,
               "resample_coeffs: bad argument");
   DFD_REQUIRE(filter == DFD_FILTER_BILINEAR || filter == DFD_FILTER_BICUBIC, DFD_ERR_UNSUPPORTED,
@@ -505,21 +494,14 @@ extern "C" DFD_API int64_t dfd_gray256_scratch_bytes(int B, int H, int W) {
   return (int64_t)B * (2 * hw + dfd::kTiles * dfd::kTiles * 256 + (int64_t)H * dfd::kOut);
 }
 
-extern "C" DFD_API int dfd_gray256(const void* rgb_u8, int B, int H, int W, int clahe, const int32_t* xmin_w,
-                                   const int32_t* count_w, const int32_t* kk_w, int ksize_w, const int32_t* xmin_h,
-                                   const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch,
-                                   float* gray256, void* stream) {
-  return dfd_gray256_strided(rgb_u8, 0, 0, B, H, W, clahe, xmin_w, count_w, kk_w, ksize_w, xmin_h, count_h, kk_h, ksize_h, scratch,
-                             gray256, stream);
-}
-
-// The same for rectangles of larger images: the crop's rows are row_stride bytes apart and consecutive crops image_stride bytes
-// (0 / 0 = dense [B,H,W,3]).  A crop of a resident image is (base + (y0·W_img + x0)·3, row_stride = W_img·3): the views of
-// detect_core / the patch grid are produced from ONE upload of the original without a copy per view.
-extern "C" DFD_API int dfd_gray256_strided(const void* rgb_u8, int64_t row_stride, int64_t image_stride, int B, int H, int W,
-                                           int clahe, const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w,
-                                           int ksize_w, const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h,
-                                           int ksize_h, void* scratch, float* gray256, void* stream) {
+// The source may be a rectangle of a larger image: the crop's rows are row_stride bytes apart and consecutive crops
+// image_stride bytes (0 / 0 = dense [B,H,W,3]).  A crop of a resident image is (base + (y0·W_img + x0)·3,
+// row_stride = W_img·3): the views of detect_core / the patch grid are produced from ONE upload of the original without a
+// copy per view.
+extern "C" DFD_API int dfd_gray256(const void* rgb_u8, int64_t row_stride, int64_t image_stride, int B, int H, int W,
+                                   int clahe, const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w,
+                                   int ksize_w, const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h,
+                                   int ksize_h, void* scratch, float* gray256, void* stream) {
   using namespace dfd;
   if (row_stride == 0) row_stride = (int64_t)W * 3;
   if (image_stride == 0) image_stride = (int64_t)H * row_stride;
@@ -530,7 +512,8 @@ extern "C" DFD_API int dfd_gray256_strided(const void* rgb_u8, int64_t row_strid
   DFD_REQUIRE(B > 0 && H > 0 && W > 0 && B <= 65535 && H <= 65535, DFD_ERR_SHAPE, "gray256: bad shape");
   DFD_REQUIRE(xmin_w && count_w && kk_w && xmin_h && count_h && kk_h, DFD_ERR_BAD_ARG,
               "gray256: resample tables missing");
-  DFD_REQUIRE(ksize_w == resample_ksize(W, kOut) && ksize_h == resample_ksize(H, kOut), DFD_ERR_BAD_ARG,
+  DFD_REQUIRE(ksize_w == resample_ksize(W, kOut, DFD_FILTER_BICUBIC) && ksize_h == resample_ksize(H, kOut, DFD_FILTER_BICUBIC),
+              DFD_ERR_BAD_ARG,
               "gray256: resample tables were built for another size");
   DFD_REQUIRE((uintptr_t)scratch % 4 == 0, DFD_ERR_BAD_ARG, "gray256: scratch must be 4-byte aligned");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -551,31 +534,21 @@ extern "C" DFD_API int dfd_gray256_strided(const void* rgb_u8, int64_t row_strid
   int launches = 1;
   const uint8_t* src = L;
   if (clahe) {
-    int tw, th;
-    if (W % kTiles == 0 && H % kTiles == 0) {
-      tw = W / kTiles;
-      th = H / kTiles;
-    } else {
-      tw = (W + (kTiles - W % kTiles)) / kTiles;
-      th = (H + (kTiles - H % kTiles)) / kTiles;
-    }
-    const int area = tw * th;
-    const float lut_scale = 255.0f / (float)area;
-    int clip = (int)(2.0 * area / 256);
-    if (clip < 1) clip = 1;
+    const ClaheGeometry g = clahe_geometry(H, W);
     // tiles that divide the image and are whole words wide (384², 224², ...): the warp-per-tile / band kernels; images are packed
     // back to back, so every row start is word aligned when W % 4 == 0
-    const bool fast = (W % kTiles == 0) && (H % kTiles == 0) && (tw % 4 == 0) && ((uintptr_t)scratch % 8 == 0);
+    const bool fast = (W % kTiles == 0) && (H % kTiles == 0) && (g.tw % 4 == 0) && ((uintptr_t)scratch % 8 == 0);
     if (fast) {
-      clahe_lut_rows_kernel<<<dim3(kTiles, B), 256, 0, st>>>(L, luts, H, W, tw, th, clip, lut_scale);
+      clahe_lut_rows_kernel<<<dim3(kTiles, B), 256, 0, st>>>(L, luts, H, W, g.tw, g.th, g.clip, g.lut_scale);
       DFD_LAUNCH_CHECK();
-      clahe_apply_band_kernel<<<dim3(kTiles + 1, B), 256, 0, st>>>(L, luts, C, H, W, th, 1.0f / (float)tw, 1.0f / (float)th);
+      clahe_apply_band_kernel<<<dim3(kTiles + 1, B), 256, 0, st>>>(L, luts, C, H, W, g.th, 1.0f / (float)g.tw,
+                                                                   1.0f / (float)g.th);
       DFD_LAUNCH_CHECK();
     } else {
-      clahe_lut_kernel<<<dim3(kTiles * kTiles, B), 256, 0, st>>>(L, luts, H, W, 1, tw, th, clip, lut_scale);
+      clahe_lut_kernel<<<dim3(kTiles * kTiles, B), 256, 0, st>>>(L, luts, H, W, 1, g.tw, g.th, g.clip, g.lut_scale);
       DFD_LAUNCH_CHECK();
-      clahe_apply_kernel<<<dim3((W + 255) / 256, H, B), 256, 0, st>>>(L, luts, C, H, W, 1, 1.0f / (float)tw,
-                                                                    1.0f / (float)th);
+      clahe_apply_kernel<<<dim3((W + 255) / 256, H, B), 256, 0, st>>>(L, luts, C, H, W, 1, 1.0f / (float)g.tw,
+                                                                    1.0f / (float)g.th);
       DFD_LAUNCH_CHECK();
     }
     launches += 2;
@@ -587,12 +560,12 @@ extern "C" DFD_API int dfd_gray256_strided(const void* rgb_u8, int64_t row_strid
     resample_rows_fast_kernel<<<dim3((H + kRowsPerCta - 1) / kRowsPerCta, B), kOut, kRowsPerCta * W, st>>>(src, rows, H, W, xmin_w,
                                                                                                             count_w, kk_w, ksize_w);
   else
-    resample_rows_kernel<<<dim3(H, B), kOut, 0, st>>>(src, rows, H, W, xmin_w, count_w, kk_w, ksize_w);
+    resize_rows_kernel<<<dim3(1, H, B), kOut, 0, st>>>(src, W, (int64_t)H * W, rows, H, kOut, 1, xmin_w, count_w, kk_w, ksize_w);
   DFD_LAUNCH_CHECK();
   if (ksize_h <= kTapMax && (uintptr_t)gray256 % 16 == 0)   // float4 stores
     resample_cols_fast_kernel<<<dim3(kOut / 16, B), 256, 0, st>>>(rows, gray256, H, xmin_h, count_h, kk_h, ksize_h);
   else
-    resample_cols_kernel<<<dim3(kOut, B), kOut, 0, st>>>(rows, gray256, H, xmin_h, count_h, kk_h, ksize_h);
+    resize_cols_kernel<<<dim3(1, kOut, B), kOut, 0, st>>>(rows, gray256, H, kOut, kOut, xmin_h, count_h, kk_h, ksize_h);
   DFD_LAUNCH_CHECK();
   g_launches.fetch_add(launches + 2, std::memory_order_relaxed);
   return DFD_OK;
@@ -614,25 +587,14 @@ extern "C" DFD_API int dfd_clahe_u8(const void* src, int B, int H, int W, int C,
   DFD_REQUIRE(B > 0 && H > 0 && W > 0 && (C == 1 || C == 3), DFD_ERR_SHAPE, "clahe: bad shape (B, H, W > 0; C = 1 or 3)");
   DFD_REQUIRE((int64_t)B * C <= 65535 && H <= 65535, DFD_ERR_SHAPE, "clahe: B*C and H must be <= 65535");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  int tw, th;
-  if (W % kTiles == 0 && H % kTiles == 0) {
-    tw = W / kTiles;
-    th = H / kTiles;
-  } else {
-    tw = (W + (kTiles - W % kTiles)) / kTiles;
-    th = (H + (kTiles - H % kTiles)) / kTiles;
-  }
-  const int area = tw * th;
-  const float lut_scale = 255.0f / (float)area;
-  int clip = (int)(2.0 * area / 256);
-  if (clip < 1) clip = 1;
+  const ClaheGeometry g = clahe_geometry(H, W);
   uint8_t* luts = reinterpret_cast<uint8_t*>(scratch);
-  clahe_lut_kernel<<<dim3(kTiles * kTiles, B * C), 256, 0, st>>>(reinterpret_cast<const uint8_t*>(src), luts, H, W, C, tw, th,
-                                                                clip, lut_scale);
+  clahe_lut_kernel<<<dim3(kTiles * kTiles, B * C), 256, 0, st>>>(reinterpret_cast<const uint8_t*>(src), luts, H, W, C, g.tw,
+                                                                g.th, g.clip, g.lut_scale);
   DFD_LAUNCH_CHECK();
   clahe_apply_kernel<<<dim3((W + 255) / 256, H, B * C), 256, 0, st>>>(reinterpret_cast<const uint8_t*>(src), luts,
                                                                      reinterpret_cast<uint8_t*>(dst), H, W, C,
-                                                                     1.0f / (float)tw, 1.0f / (float)th);
+                                                                     1.0f / (float)g.tw, 1.0f / (float)g.th);
   DFD_LAUNCH_CHECK();
   g_launches.fetch_add(2, std::memory_order_relaxed);
   return DFD_OK;
@@ -641,19 +603,11 @@ extern "C" DFD_API int dfd_clahe_u8(const void* src, int B, int H, int W, int C,
 // Pillow Image.resize((OW, OH), BILINEAR | BICUBIC) for batches of same-size 8-bit images, 1 or 3 interleaved channels:
 // what torchvision's transforms.Resize does to a PIL image (inference_ai_human_images.py:200-204,
 // train_fusion_head_only.py:67-74) — horizontal pass, u8, vertical pass.  scratch: B*H*OW*C bytes.
-extern "C" DFD_API int dfd_resize_u8(const void* src, int B, int H, int W, int C, int OH, int OW, const int32_t* xmin_w,
-                                     const int32_t* count_w, const int32_t* kk_w, int ksize_w, const int32_t* xmin_h,
-                                     const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch, void* dst,
-                                     void* stream) {
-  return dfd_resize_u8_strided(src, 0, 0, B, H, W, C, OH, OW, xmin_w, count_w, kk_w, ksize_w, xmin_h, count_h, kk_h, ksize_h,
-                               scratch, dst, stream);
-}
-
-// The same for rectangles of larger images (strides in bytes; 0 / 0 = dense), see dfd_gray256_strided.
-extern "C" DFD_API int dfd_resize_u8_strided(const void* src, int64_t row_stride, int64_t image_stride, int B, int H, int W, int C,
-                                             int OH, int OW, const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w,
-                                             int ksize_w, const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h,
-                                             int ksize_h, void* scratch, void* dst, void* stream) {
+// The source may be a rectangle of a larger image (strides in bytes; 0 / 0 = dense), see dfd_gray256.
+extern "C" DFD_API int dfd_resize_u8(const void* src, int64_t row_stride, int64_t image_stride, int B, int H, int W, int C,
+                                     int OH, int OW, const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w,
+                                     int ksize_w, const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h,
+                                     int ksize_h, void* scratch, void* dst, void* stream) {
   using namespace dfd;
   if (row_stride == 0) row_stride = (int64_t)W * C;
   if (image_stride == 0) image_stride = (int64_t)H * row_stride;

@@ -298,9 +298,8 @@ class SiglipEngine:
         """Per kernel family, summed over every forward since the last read: {'gemm': (ms, launches), 'attention': ...,
         'layernorm': ..., 'patchify': ..., 'map_attention': ...}; with by_gemm_type also 'gemm_qkv' / 'gemm_out' / 'gemm_fc1' /
         'gemm_fc2' / 'gemm_other' (patch embedding + pooling head), which add up to 'gemm'.  Waits for the last recorded launch."""
-        n = 9
-        ms, cnt = (C.c_float * n)(), (C.c_int * n)()
-        check(self._lib.dfd_engine_profile_read_families(self._h, n, ms, cnt))
+        ms, cnt = (C.c_float * 9)(), (C.c_int * 9)()
+        check(self._lib.dfd_engine_profile_read(self._h, ms, cnt))
         out = {k: (float(ms[i]), int(cnt[i])) for i, k in enumerate(self.FAMILIES)}
         gm = [0, 5, 6, 7, 8]
         out["gemm"] = (float(sum(ms[i] for i in gm)), int(sum(cnt[i] for i in gm)))

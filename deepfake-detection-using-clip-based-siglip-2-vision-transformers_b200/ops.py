@@ -43,7 +43,7 @@ def gemm_bf16(a: torch.Tensor, w: torch.Tensor, *, bias=None, act: int = 0, pos=
     """out[M,N] = epilogue(a[M,K] @ w[N,K].T); bf16 in/out, fp32 accumulate in TMEM (dfd_gemm_bf16).
     act: 0 none, 1 gelu_tanh, 2 gelu_erf, 3 sigmoid; residual_op: 0 add, 1 multiply.
     stats_out: fp32 [ceil(N/64), M, 2] per-chunk (sum, sum of squares) of the bf16 output rows (written, not
-    accumulated); ln_rowstats: fp32 [M, 2] (rowstats_bf16) or [parts, M, 2] partials (a previous GEMM's stats_out)."""
+    accumulated); ln_rowstats: fp32 [M, 2] whole-row sums or [parts, M, 2] partials (a previous GEMM's stats_out)."""
     _need_cuda(a, w, bias, pos, residual, out)
     assert a.dtype == torch.bfloat16 and w.dtype == torch.bfloat16
     assert a.dim() == 2 and w.dim() == 2 and a.shape[1] == w.shape[1]
@@ -69,7 +69,6 @@ def gemm_bf16(a: torch.Tensor, w: torch.Tensor, *, bias=None, act: int = 0, pos=
     # two-bf16 residual stream: residual_lo (tiled, ops.lo_to_tiled) is read with the residual and rewritten in place with the
     # low half of the new value (see dfd_gemm_epilogue.residual_lo)
     epi.residual_lo = _p(residual_lo)
-    epi.ldlo = 0
     if residual_lo is not None:
         assert residual_lo.dtype == torch.bfloat16 and residual_lo.is_contiguous() and \
             tuple(residual_lo.shape) == ((M + 127) // 128, (N + 63) // 64, 8, 128, 8), "residual_lo: see ops.lo_to_tiled"
@@ -105,29 +104,27 @@ def lo_from_tiled(t: torch.Tensor, M: int, N: int) -> torch.Tensor:
     return t.permute(0, 3, 1, 2, 4).reshape(mb * 128, nc * 64)[:M, :N].contiguous()
 
 
-def layernorm_bf16(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float = 1e-6) -> torch.Tensor:
-    _need_cuda(x, gamma, beta)
+def layernorm_bf16(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float = 1e-6,
+                   lo: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """LayerNorm of the bf16 rows of x (dfd_layernorm_bf16); with lo (tiled, ops.lo_to_tiled) of the two-bf16 rows x + lo."""
+    _need_cuda(x, gamma, beta, lo)
     assert x.dtype == torch.bfloat16 and x.dim() == 2 and x.stride(1) == 1
     assert gamma.dtype == torch.float32 and beta.dtype == torch.float32
+    M, D = x.shape
+    if lo is not None:
+        assert lo.dtype == torch.bfloat16 and lo.is_contiguous() and \
+            tuple(lo.shape) == ((M + 127) // 128, (D + 63) // 64, 8, 128, 8), "lo: see ops.lo_to_tiled"
     y = torch.empty_like(x)
-    check(_lib.load().dfd_layernorm_bf16(x.data_ptr(), x.stride(0), y.data_ptr(), y.stride(0), gamma.data_ptr(),
-                                         beta.data_ptr(), x.shape[0], x.shape[1], eps, current_stream()))
+    check(_lib.load().dfd_layernorm_bf16(x.data_ptr(), x.stride(0), _p(lo), y.data_ptr(), y.stride(0), gamma.data_ptr(),
+                                         beta.data_ptr(), M, D, eps, current_stream()))
     return y
-
-
-def rowstats_bf16(x: torch.Tensor) -> torch.Tensor:
-    _need_cuda(x)
-    assert x.dtype == torch.bfloat16 and x.dim() == 2 and x.stride(1) == 1
-    st = torch.empty((x.shape[0], 2), dtype=torch.float32, device=x.device)
-    check(_lib.load().dfd_rowstats_bf16(x.data_ptr(), x.stride(0), st.data_ptr(), x.shape[0], x.shape[1],
-                                        current_stream()))
-    return st
 
 
 def attention_bf16(qkv: torch.Tensor, B: int, N: int, H: int, hd: int, scale: Optional[float] = None,
                    impl: Optional[int] = None) -> torch.Tensor:
     """qkv [B*N, 3*H*hd] (q | k | v) -> [B*N, H*hd]; non-causal softmax(q k^T scale) v.
-    impl None = product dispatch; 5 / 2 force the dual-query-tile / single-tile persistent tcgen05 kernel (A/B tests)."""
+    impl None = product dispatch (2 for N <= 128, 5 above); 5 / 2 force the dual-query-tile / single-tile persistent
+    tcgen05 kernel for any N (A/B tests); any other value is rejected (DFD_ERR_BAD_ARG)."""
     _need_cuda(qkv)
     assert qkv.dtype == torch.bfloat16 and qkv.shape == (B * N, 3 * H * hd) and qkv.stride(1) == 1
     out = torch.empty((B * N, H * hd), dtype=torch.bfloat16, device=qkv.device)
@@ -267,16 +264,16 @@ FILTERS = {"bilinear": 2, "bicubic": 3}   # PIL.Image.BILINEAR / BICUBIC
 
 
 def resample_coeffs(in_size: int, out_size: int = 256, filter: str = "bicubic"):
-    """Pillow's 8bpc resample tables for one axis (host, dfd_resample_coeffs_filter_host): (xmin, count, kk) int32
+    """Pillow's 8bpc resample tables for one axis (host, dfd_resample_coeffs_host): (xmin, count, kk) int32
     numpy arrays, kk [out_size, ksize].  Works without a GPU."""
     import numpy as np
 
     lib = _lib.load()
     f = FILTERS[filter]
-    ks = lib.dfd_resample_ksize_filter(in_size, out_size, f)
+    ks = lib.dfd_resample_ksize(in_size, out_size, f)
     xmin, cnt = np.zeros(out_size, np.int32), np.zeros(out_size, np.int32)
     kk = np.zeros((out_size, ks), np.int32)
-    check(lib.dfd_resample_coeffs_filter_host(in_size, out_size, f, xmin.ctypes.data, cnt.ctypes.data, kk.ctypes.data))
+    check(lib.dfd_resample_coeffs_host(in_size, out_size, f, xmin.ctypes.data, cnt.ctypes.data, kk.ctypes.data))
     return xmin, cnt, kk
 
 
@@ -311,9 +308,9 @@ def resize_u8(images: torch.Tensor, out_h: int, out_w: int, filter: str = "bilin
     xh, ch, kh = _resample_tables(H, images.device, out_h, filter)
     scratch = torch.empty((B, H, out_w, C), dtype=torch.uint8, device=images.device)
     out = torch.empty((B, out_h, out_w, C), dtype=torch.uint8, device=images.device)
-    check(_lib.load().dfd_resize_u8_strided(images.data_ptr(), rs, ims, B, H, W, C, out_h, out_w, xw.data_ptr(), cw.data_ptr(),
-                                            kw.data_ptr(), kw.shape[1], xh.data_ptr(), ch.data_ptr(), kh.data_ptr(), kh.shape[1],
-                                            scratch.data_ptr(), out.data_ptr(), current_stream()))
+    check(_lib.load().dfd_resize_u8(images.data_ptr(), rs, ims, B, H, W, C, out_h, out_w, xw.data_ptr(), cw.data_ptr(),
+                                    kw.data_ptr(), kw.shape[1], xh.data_ptr(), ch.data_ptr(), kh.data_ptr(), kh.shape[1],
+                                    scratch.data_ptr(), out.data_ptr(), current_stream()))
     return out
 
 
@@ -334,7 +331,7 @@ def clahe_u8(images: torch.Tensor) -> torch.Tensor:
 def gray256_from_rgb(images: torch.Tensor, clahe: bool, scratch: Optional[torch.Tensor] = None,
                      out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """u8 RGB images [B,H,W,3] (NHWC, device; dense or a rectangle view of a larger image) -> gray256 f32 [B,256,256] in [0,1]
-    (dfd_gray256[_strided]): Pillow 'L' luma, optional OpenCV CLAHE(2.0, 8x8), Pillow bicubic resize, /255 —
+    (dfd_gray256): Pillow 'L' luma, optional OpenCV CLAHE(2.0, 8x8), Pillow bicubic resize, /255 —
     train_fusion_head_only.py:142-148 (clahe=True), deepfake-detector-v2/app.py:736-749.  EXIF orientation is the decoder's
     business (apply ImageOps.exif_transpose before handing pixels over, as the reference does)."""
     _need_cuda(images)
@@ -349,9 +346,9 @@ def gray256_from_rgb(images: torch.Tensor, clahe: bool, scratch: Optional[torch.
     xh, ch, kh = _resample_tables(H, images.device)
     if out is None:
         out = torch.empty((B, 256, 256), dtype=torch.float32, device=images.device)
-    check(lib.dfd_gray256_strided(images.data_ptr(), rs, ims, B, H, W, int(clahe), xw.data_ptr(), cw.data_ptr(), kw.data_ptr(),
-                                  kw.shape[1], xh.data_ptr(), ch.data_ptr(), kh.data_ptr(), kh.shape[1], scratch.data_ptr(),
-                                  out.data_ptr(), current_stream()))
+    check(lib.dfd_gray256(images.data_ptr(), rs, ims, B, H, W, int(clahe), xw.data_ptr(), cw.data_ptr(), kw.data_ptr(),
+                          kw.shape[1], xh.data_ptr(), ch.data_ptr(), kh.data_ptr(), kh.shape[1], scratch.data_ptr(),
+                          out.data_ptr(), current_stream()))
     return out
 
 

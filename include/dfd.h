@@ -81,14 +81,13 @@ typedef struct dfd_gemm_epilogue {
   float ln_eps;
   float* stats_out;          /* [ceil(N/64)][M][2] fp32 partials (see above), or NULL */
   int residual_op;           /* 0: v += residual (default), 1: v *= residual (gating: Siglip2sidafrozen.py:737) */
-  int ln_parts;              /* partial pairs per row in ln_rowstats; 0 or 1 = plain [M,2] (dfd_rowstats_bf16) */
+  int ln_parts;              /* partial pairs per row in ln_rowstats; 0 or 1 = one [M,2] pair per row (whole-row sums) */
   void* residual_lo;         /* bf16 or NULL: low half of a two-bf16 residual stream.  With it the epilogue value is
                               * v = ... + residual + residual_lo (read only when residual is given), C = hi = bf16(v) and
                               * residual_lo = bf16(v - hi) is written back (in place), so the stream carries ~16 mantissa bits
                               * across layers like the fp32 residual of the reference's autocast path.  Layout (private to the
-                              * epilogue and dfd_layernorm2_bf16, coalesced for the epilogue's row-per-lane mapping):
+                              * epilogue and dfd_layernorm_bf16, coalesced for the epilogue's row-per-lane mapping):
                               * [ceil(M/128)][ceil(N/64)][8][128][8] = (row block, 64-column chunk, 8-column group, row, column) */
-  int64_t ldlo;              /* unused */
 } dfd_gemm_epilogue;
 
 /* C[M,N] (bf16) = epi(A[M,K] (bf16, lda) · W[N,K]ᵀ (bf16, ldw)), fp32 accumulate in TMEM.
@@ -113,14 +112,10 @@ DFD_API int dfd_gemm_last_variant(void);
 DFD_API int64_t dfd_gemm_variant_launches(int variant);
 
 /* y[M,D] (bf16) = LayerNorm(x[M,D] (bf16)) · gamma + beta, fp32 statistics, eps as given.
- * HF:modeling_siglip.py:348,357 (layer_norm1/2), :618 (post_layernorm). */
-DFD_API int dfd_layernorm_bf16(const void* x, int64_t ldx, void* y, int64_t ldy, const float* gamma,
+ * HF:modeling_siglip.py:348,357 (layer_norm1/2), :618 (post_layernorm).  lo = NULL: the rows are x alone; otherwise
+ * they are the two-bf16 sum x + lo, lo in the tiled layout of dfd_gemm_epilogue.residual_lo. */
+DFD_API int dfd_layernorm_bf16(const void* x, int64_t ldx, const void* lo, void* y, int64_t ldy, const float* gamma,
                                const float* beta, int M, int D, float eps, void* stream);
-/* The same over the two-bf16 row x + lo, lo in the tiled layout of dfd_gemm_epilogue.residual_lo (ldlo unused). */
-DFD_API int dfd_layernorm2_bf16(const void* x, int64_t ldx, const void* lo, int64_t ldlo, void* y, int64_t ldy,
-                                const float* gamma, const float* beta, int M, int D, float eps, void* stream);
-/* stats[M,2] = (Σx, Σx²) of bf16 rows (feeds the LN-folded GEMM epilogue when the producer was not a GEMM). */
-DFD_API int dfd_rowstats_bf16(const void* x, int64_t ldx, float* stats, int M, int D, void* stream);
 
 /* Non-causal multi-head attention over packed qkv[B·N, 3·H·hd] (bf16; q | k | v column blocks, head h at
  * columns h·hd) -> out[B·N, H·hd] (bf16).  softmax(q·kᵀ·scale) in fp32.
@@ -201,41 +196,31 @@ DFD_API int64_t dfd_freq_scratch_bytes(int B);
  * cv2.createCLAHE(2.0,(8,8)).apply -> Pillow resize((256,256), BICUBIC) (22-bit fixed-point antialiased resample,
  * horizontal pass then vertical, u8 in between) -> /255.  Bit-exact with Pillow 12.2 / OpenCV 4.13 (oracle/gray_ref.py).
  * The per-axis coefficient tables are built on the HOST by dfd_resample_coeffs_host (double precision, Pillow's
- * precompute_coeffs + normalize_coeffs_8bpc; no GPU needed) and passed as device arrays: xmin[256], count[256],
- * kk[256][ksize] with ksize = dfd_resample_ksize(in_size, 256).  scratch: dfd_gray256_scratch_bytes(B,H,W). */
-DFD_API int dfd_resample_ksize(int in_size, int out_size);
-DFD_API int dfd_resample_coeffs_host(int in_size, int out_size, int32_t* xmin_host, int32_t* count_host,
+ * precompute_coeffs + normalize_coeffs_8bpc; no GPU needed) and passed as device arrays: xmin[out], count[out],
+ * kk[out][ksize] with ksize = dfd_resample_ksize(in_size, out, filter); gray256 takes BICUBIC tables with out = 256.
+ * scratch: dfd_gray256_scratch_bytes(B,H,W). */
+enum { DFD_FILTER_BILINEAR = 2, DFD_FILTER_BICUBIC = 3 };   /* PIL.Image.BILINEAR / BICUBIC */
+DFD_API int dfd_resample_ksize(int in_size, int out_size, int filter);
+DFD_API int dfd_resample_coeffs_host(int in_size, int out_size, int filter, int32_t* xmin_host, int32_t* count_host,
                                      int32_t* kk_host);
 DFD_API int64_t dfd_gray256_scratch_bytes(int B, int H, int W);
 
 /* Pillow Image.resize((OW,OH), BILINEAR|BICUBIC) for a batch of same-size 8-bit images with 1 or 3 interleaved channels
  * — what torchvision transforms.Resize((S,S)) does to the PIL image in the reference's preprocess
  * (inference_ai_human_images.py:200-204, train_fusion_head_only.py:67-74) and what open_clip's preprocess does with
- * BICUBIC.  Same fixed-point arithmetic as above, bit-exact; tables from dfd_resample_coeffs_filter_host with
- * ksize = dfd_resample_ksize_filter(in, out, filter).  scratch: B*H*OW*C bytes. */
-enum { DFD_FILTER_BILINEAR = 2, DFD_FILTER_BICUBIC = 3 };   /* PIL.Image.BILINEAR / BICUBIC */
-DFD_API int dfd_resample_ksize_filter(int in_size, int out_size, int filter);
-DFD_API int dfd_resample_coeffs_filter_host(int in_size, int out_size, int filter, int32_t* xmin_host,
-                                            int32_t* count_host, int32_t* kk_host);
-/* Strided forms of dfd_resize_u8 / dfd_gray256: the source is a rectangle of a larger image — rows row_stride bytes apart,
- * consecutive rectangles image_stride bytes apart (0 / 0 = dense).  A crop (x0, y0, w, h) of a resident u8 RGB image of width Wi is
+ * BICUBIC.  Same fixed-point arithmetic as above, bit-exact; tables from dfd_resample_coeffs_host with the same filter.
+ * scratch: B*H*OW*C bytes.
+ * dfd_resize_u8 and dfd_gray256 read a rectangle of a larger image — rows row_stride bytes apart, consecutive rectangles
+ * image_stride bytes apart (0 / 0 = dense).  A crop (x0, y0, w, h) of a resident u8 RGB image of width Wi is
  * (base + (y0·Wi + x0)·3, row_stride = Wi·3): the multicrop views of detect_core (deepfake-detector-v2/app.py:1418-1430,
  * appv3.py:3315-3350) and the patch-grid cells (:1461-1485) come from one upload, without a copy per view. */
-DFD_API int dfd_resize_u8_strided(const void* src, int64_t row_stride, int64_t image_stride, int B, int H, int W, int C, int OH,
-                                  int OW, const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w, int ksize_w,
-                                  const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch,
-                                  void* dst, void* stream);
-DFD_API int dfd_gray256_strided(const void* rgb_u8, int64_t row_stride, int64_t image_stride, int B, int H, int W, int clahe,
-                                const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w, int ksize_w,
-                                const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch,
-                                float* gray256, void* stream);
-DFD_API int dfd_resize_u8(const void* src, int B, int H, int W, int C, int OH, int OW, const int32_t* xmin_w,
-                          const int32_t* count_w, const int32_t* kk_w, int ksize_w, const int32_t* xmin_h,
-                          const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch, void* dst,
-                          void* stream);
-DFD_API int dfd_gray256(const void* rgb_u8, int B, int H, int W, int clahe, const int32_t* xmin_w,
-                        const int32_t* count_w, const int32_t* kk_w, int ksize_w, const int32_t* xmin_h,
-                        const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch,
+DFD_API int dfd_resize_u8(const void* src, int64_t row_stride, int64_t image_stride, int B, int H, int W, int C, int OH,
+                          int OW, const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w, int ksize_w,
+                          const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch,
+                          void* dst, void* stream);
+DFD_API int dfd_gray256(const void* rgb_u8, int64_t row_stride, int64_t image_stride, int B, int H, int W, int clahe,
+                        const int32_t* xmin_w, const int32_t* count_w, const int32_t* kk_w, int ksize_w,
+                        const int32_t* xmin_h, const int32_t* count_h, const int32_t* kk_h, int ksize_h, void* scratch,
                         float* gray256 /*[B,256,256]*/, void* stream);
 
 /* Per-channel CLAHE of dense u8 images [B,H,W,C] (C = 1 or 3): cv2.createCLAHE(clipLimit=2.0, tileGridSize=(8,8)).apply on
@@ -358,12 +343,10 @@ DFD_API int64_t dfd_engine_workspace_bytes(const dfd_engine* e);
 /* Measurement aid (bench.py roofline): dfd_engine_profile(e, n) with n > 0 makes dfd_engine_forward bracket every launch
  * with CUDA events on the caller's stream, with room for n forwards (launches past that are not recorded); n = 0 switches
  * it off.  dfd_engine_profile_read waits for the last recorded event, sums the durations recorded since the previous read
- * per kernel family (ms4/count4 index: 0 GEMM, 1 attention, 2 LayerNorm, 3 other) and clears the record. */
+ * per kernel family and clears the record.  ms[9] / count[9] index: 0 GEMM (patch embedding, pooling head), 1 attention,
+ * 2 LayerNorm, 3 patchify, 4 MAP attention, 5 qkv GEMM, 6 out-projection GEMM, 7 fc1 GEMM, 8 fc2 GEMM. */
 DFD_API int dfd_engine_profile(dfd_engine* e, int forwards);
-DFD_API int dfd_engine_profile_read(dfd_engine* e, float* ms4, int* count4);
-/* Same with n families: 0 GEMM (patch embedding, pooling head; with n <= 5 also the encoder GEMMs), 1 attention, 2 LayerNorm,
- * 3 patchify, 4 MAP attention, 5 qkv GEMM, 6 out-projection GEMM, 7 fc1 GEMM, 8 fc2 GEMM (families >= n fold into n - 1). */
-DFD_API int dfd_engine_profile_read_families(dfd_engine* e, int n, float* ms, int* count);
+DFD_API int dfd_engine_profile_read(dfd_engine* e, float* ms, int* count);
 
 #ifdef __cplusplus
 }

@@ -70,7 +70,7 @@ def attention(B, arch):
     N, H, hd = arch.tokens, arch.num_attention_heads, arch.head_dim
     qkv = torch.randn(B * N, 3 * H * hd, device=DEV).to(torch.bfloat16)
     fl = 4.0 * N * N * H * hd * B
-    for impl in (2, 5, 6, 7):
+    for impl in (2, 5):
         med, best = timeit(lambda: ops.attention_bf16(qkv, B, N, H, hd, impl=impl))
         print(f"attention impl={impl} B={B} N={N} H={H} hd={hd}: {med:8.3f} ms {fl / med / 1e9:7.1f} TF/s best {best:.3f}", flush=True)
     try:
@@ -105,7 +105,6 @@ def memory_bound(B, arch):
     x = torch.randn(B * N, D, device=DEV).to(torch.bfloat16)
     g = torch.ones(D, device=DEV)
     line(f"layernorm M={B * N} D={D}", x.numel() * 4, lambda: ops.layernorm_bf16(x, g, g))
-    line(f"rowstats M={B * N} D={D}", x.numel() * 2, lambda: ops.rowstats_bf16(x))
     kv = torch.randn(B * N, 2 * D, device=DEV).to(torch.bfloat16)
     q = torch.randn(D, device=DEV)
     line(f"map_attention B={B} N={N}", kv.numel() * 2, lambda: ops.map_attention_bf16(kv, q, B, N, H, D // H))

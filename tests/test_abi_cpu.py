@@ -327,7 +327,7 @@ def test_fused_normalise_rounds_to_the_reference_bf16_for_every_byte():
 
 def test_tiled_layout_of_the_low_halves_round_trips():
     """ops.lo_to_tiled / lo_from_tiled: the [row block][64-column chunk][8-column group][row][8] order the GEMM epilogue and
-    dfd_layernorm2_bf16 address (element (r, c) at (((r/128·nch + c/64)·8 + (c%64)/8)·128 + r%128)·8 + c%8)."""
+    dfd_layernorm_bf16 address (element (r, c) at (((r/128·nch + c/64)·8 + (c%64)/8)·128 + r%128)·8 + c%8)."""
     import torch
 
     from dfd import ops
