@@ -159,17 +159,84 @@ def _gelu_tanh(x):
     return 0.5 * x * (1.0 + torch.tanh(math.sqrt(2.0 / math.pi) * (x + 0.044715 * x ** 3)))
 
 
-def _mha(q, k, v, H, ac):
-    """q [B,Nq,D], k/v [B,Nk,D] -> [B,Nq,D]; softmax in fp32; P and the output round to bf16 under autocast."""
+def _mha(q, k, v, H, ac, scale=None):
+    """q [B,Nq,D], k/v [B,Nk,D] -> [B,Nq,D]; softmax in fp32; P and the output round to bf16 under autocast.
+    scale: the logit scale, 1/sqrt(head dim) unless given."""
     B, Nq, D = q.shape
     hd = D // H
     qh = _rb(q, ac).view(B, Nq, H, hd).transpose(1, 2)
     kh = _rb(k, ac).view(B, -1, H, hd).transpose(1, 2)
     vh = _rb(v, ac).view(B, -1, H, hd).transpose(1, 2)
-    s = (qh @ kh.transpose(-1, -2)) * (hd ** -0.5)
+    s = (qh @ kh.transpose(-1, -2)) * (hd ** -0.5 if scale is None else scale)
     p = torch.softmax(s, dim=-1)
     o = _rb(p, ac) @ vh
     return _rb(o.transpose(1, 2).reshape(B, Nq, D), ac)
+
+
+def _check_mode(mode: str) -> bool:
+    assert mode in ("fp32", "autocast")
+    return mode == "autocast"
+
+
+# The three stages below compute in the dtype of their inputs (float32, or float64 with a float64 state dict),
+# so mode="fp32" on float64 tensors is a float64 reference of the same arithmetic.
+@torch.no_grad()
+def embed(sd: dict, c: VisionConfig, pixel_values: torch.Tensor, mode: str = "fp32") -> torch.Tensor:
+    """pixel_values [B,3,S,S] (already normalised) -> hidden_states[0] [B,N,D]: patch embedding + position."""
+    ac = _check_mode(mode)
+    B = pixel_values.shape[0]
+    P, G, D = c.patch_size, c.grid, c.hidden_size
+    # conv k=s=P, padding valid == im2col over the top-left G*P x G*P crop, column order (c, ky, kx)
+    x = pixel_values[:, :, : G * P, : G * P]
+    if x.dtype != torch.float64:
+        x = x.to(torch.float32)
+    patches = x.reshape(B, 3, G, P, G, P).permute(0, 2, 4, 1, 3, 5).reshape(B, G * G, 3 * P * P)
+    w = sd["embeddings.patch_embedding.weight"].reshape(D, -1)
+    h = _linear(patches, w, sd["embeddings.patch_embedding.bias"], ac)
+    return h + sd["embeddings.position_embedding.weight"][None]
+
+
+@torch.no_grad()
+def encoder_layer(sd: dict, c: VisionConfig, i: int, h: torch.Tensor, mode: str = "fp32",
+                  attn_scale: float | None = None) -> torch.Tensor:
+    """hidden_states[i] [B,N,D] -> hidden_states[i+1]: encoder layer i (pre-LN attention block, then pre-LN MLP).
+    attn_scale overrides the attention logit scale 1/sqrt(head dim) (tests use it to measure a kernel's effective scale)."""
+    ac = _check_mode(mode)
+    eps = c.layer_norm_eps
+    p = f"encoder.layers.{i}."
+    y = _layernorm(h, sd[p + "layer_norm1.weight"], sd[p + "layer_norm1.bias"], eps)
+    q = _linear(y, sd[p + "self_attn.q_proj.weight"], sd[p + "self_attn.q_proj.bias"], ac)
+    k = _linear(y, sd[p + "self_attn.k_proj.weight"], sd[p + "self_attn.k_proj.bias"], ac)
+    v = _linear(y, sd[p + "self_attn.v_proj.weight"], sd[p + "self_attn.v_proj.bias"], ac)
+    a = _mha(q, k, v, c.num_attention_heads, ac, attn_scale)
+    h = h + _linear(a, sd[p + "self_attn.out_proj.weight"], sd[p + "self_attn.out_proj.bias"], ac)
+    y = _layernorm(h, sd[p + "layer_norm2.weight"], sd[p + "layer_norm2.bias"], eps)
+    m = _rb(_gelu_tanh(_linear(y, sd[p + "mlp.fc1.weight"], sd[p + "mlp.fc1.bias"], ac)), ac)
+    return h + _linear(m, sd[p + "mlp.fc2.weight"], sd[p + "mlp.fc2.bias"], ac)
+
+
+@torch.no_grad()
+def post_layernorm(sd: dict, c: VisionConfig, h: torch.Tensor) -> torch.Tensor:
+    """hidden_states[L] -> last_hidden_state."""
+    return _layernorm(h, sd["post_layernorm.weight"], sd["post_layernorm.bias"], c.layer_norm_eps)
+
+
+@torch.no_grad()
+def map_head(sd: dict, c: VisionConfig, last: torch.Tensor, mode: str = "fp32") -> torch.Tensor:
+    """last_hidden_state [B,N,D] -> pooler_output [B,D]: MAP pooling (probe attention, LayerNorm, MLP residual)."""
+    ac = _check_mode(mode)
+    B, D = last.shape[0], c.hidden_size
+    wi, bi = sd["head.attention.in_proj_weight"], sd["head.attention.in_proj_bias"]
+    probe = sd["head.probe"].reshape(1, 1, D).expand(B, 1, D)
+    q = _linear(probe, wi[:D], bi[:D], ac)
+    k = _linear(last, wi[D : 2 * D], bi[D : 2 * D], ac)
+    v = _linear(last, wi[2 * D :], bi[2 * D :], ac)
+    a = _mha(q, k, v, c.num_attention_heads, ac)
+    r = _linear(a, sd["head.attention.out_proj.weight"], sd["head.attention.out_proj.bias"], ac)
+    y = _layernorm(r, sd["head.layernorm.weight"], sd["head.layernorm.bias"], c.layer_norm_eps)
+    m = _rb(_gelu_tanh(_linear(y, sd["head.mlp.fc1.weight"], sd["head.mlp.fc1.bias"], ac)), ac)
+    out = r + _linear(m, sd["head.mlp.fc2.weight"], sd["head.mlp.fc2.bias"], ac)
+    return out[:, 0]
 
 
 @torch.no_grad()
@@ -177,43 +244,13 @@ def siglip_vision_forward(sd: dict, c: VisionConfig, pixel_values: torch.Tensor,
                           output_hidden_states: bool = False) -> dict:
     """pixel_values f32 [B,3,S,S] (already normalised) -> {'pooler_output' [B,D], 'last_hidden_state' [B,N,D],
     'hidden_states' tuple of L+1 (optional)}."""
-    assert mode in ("fp32", "autocast")
-    ac = mode == "autocast"
-    B = pixel_values.shape[0]
-    P, G, D, H = c.patch_size, c.grid, c.hidden_size, c.num_attention_heads
-    eps = c.layer_norm_eps
-    # conv k=s=P, padding valid == im2col over the top-left G*P x G*P crop, column order (c, ky, kx)
-    x = pixel_values[:, :, : G * P, : G * P].to(torch.float32)
-    patches = x.reshape(B, 3, G, P, G, P).permute(0, 2, 4, 1, 3, 5).reshape(B, G * G, 3 * P * P)
-    w = sd["embeddings.patch_embedding.weight"].reshape(D, -1)
-    h = _linear(patches, w, sd["embeddings.patch_embedding.bias"], ac)
-    h = h + sd["embeddings.position_embedding.weight"][None]
+    h = embed(sd, c, pixel_values, mode)
     hidden = [h]
     for i in range(c.num_hidden_layers):
-        p = f"encoder.layers.{i}."
-        y = _layernorm(h, sd[p + "layer_norm1.weight"], sd[p + "layer_norm1.bias"], eps)
-        q = _linear(y, sd[p + "self_attn.q_proj.weight"], sd[p + "self_attn.q_proj.bias"], ac)
-        k = _linear(y, sd[p + "self_attn.k_proj.weight"], sd[p + "self_attn.k_proj.bias"], ac)
-        v = _linear(y, sd[p + "self_attn.v_proj.weight"], sd[p + "self_attn.v_proj.bias"], ac)
-        a = _mha(q, k, v, H, ac)
-        h = h + _linear(a, sd[p + "self_attn.out_proj.weight"], sd[p + "self_attn.out_proj.bias"], ac)
-        y = _layernorm(h, sd[p + "layer_norm2.weight"], sd[p + "layer_norm2.bias"], eps)
-        m = _rb(_gelu_tanh(_linear(y, sd[p + "mlp.fc1.weight"], sd[p + "mlp.fc1.bias"], ac)), ac)
-        h = h + _linear(m, sd[p + "mlp.fc2.weight"], sd[p + "mlp.fc2.bias"], ac)
+        h = encoder_layer(sd, c, i, h, mode)
         hidden.append(h)
-    last = _layernorm(h, sd["post_layernorm.weight"], sd["post_layernorm.bias"], eps)
-    # MAP head
-    wi, bi = sd["head.attention.in_proj_weight"], sd["head.attention.in_proj_bias"]
-    probe = sd["head.probe"].reshape(1, 1, D).expand(B, 1, D)
-    q = _linear(probe, wi[:D], bi[:D], ac)
-    k = _linear(last, wi[D : 2 * D], bi[D : 2 * D], ac)
-    v = _linear(last, wi[2 * D :], bi[2 * D :], ac)
-    a = _mha(q, k, v, H, ac)
-    r = _linear(a, sd["head.attention.out_proj.weight"], sd["head.attention.out_proj.bias"], ac)
-    y = _layernorm(r, sd["head.layernorm.weight"], sd["head.layernorm.bias"], eps)
-    m = _rb(_gelu_tanh(_linear(y, sd["head.mlp.fc1.weight"], sd["head.mlp.fc1.bias"], ac)), ac)
-    out = r + _linear(m, sd["head.mlp.fc2.weight"], sd["head.mlp.fc2.bias"], ac)
-    res = {"pooler_output": out[:, 0], "last_hidden_state": last}
+    last = post_layernorm(sd, c, h)
+    res = {"pooler_output": map_head(sd, c, last, mode), "last_hidden_state": last}
     if output_hidden_states:
         res["hidden_states"] = tuple(hidden)
     return res
