@@ -110,6 +110,8 @@ SIGNATURES = {
     "dfd_attention_bf16_impl": (_I, [_P, _L, _P, _L, _I, _I, _I, _I, _F, _I, _P]),
     "dfd_patchify": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _L, _P]),
     "dfd_map_attention_bf16": (_I, [_P, _L, _P, _P, _L, _I, _I, _I, _I, _F, _P]),
+    "dfd_attention_probs": (_I, [_P, _L, _I, _I, _I, _I, _F, _I, _P, _P]),
+    "dfd_attention_rollout": (_I, [_P, _P, _I, _I, _I, _I, _F, _I, _I, _P, _P, _P]),
     "dfd_head_fwd": (_I, [C.POINTER(HeadWeights), _P, _L, _I, _P, _P, _P, _P, _P]),
     "dfd_freq_features": (_I, [_P, _I, _P, _F, _I, _P, _P, _P]),
     "dfd_freq_scratch_bytes": (_L, [_I]),
@@ -133,6 +135,7 @@ SIGNATURES = {
     "dfd_engine_forward": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
     "dfd_engine_workspace_bytes": (_L, [_P]),
     "dfd_engine_set_hidden_tap": (_I, [_P, _P]),
+    "dfd_engine_set_attention_tap": (_I, [_P, _P, _I, _P]),
     "dfd_engine_set_graphs": (_I, [_P, _I]),
     "dfd_engine_set_precise_residual": (_I, [_P, _I]),
     "dfd_engine_graph_replays": (C.c_int64, [_P]),

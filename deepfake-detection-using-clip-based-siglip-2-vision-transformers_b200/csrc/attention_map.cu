@@ -20,10 +20,11 @@ namespace {
 // P·V pass gives each thread one chunk column and every (256 / chunks)-th key.
 constexpr int kMapThreads = 256;
 
-template <int HD>
+// kProbs: also write the probabilities probs[b, h, n] (the attention-map tap); the product instantiations have it off
+template <int HD, bool kProbs>
 __global__ void __launch_bounds__(kMapThreads)
 map_attention_kernel(const __nv_bfloat16* __restrict__ kv, int64_t ldkv, const float* __restrict__ q,
-                     __nv_bfloat16* __restrict__ out, int64_t ldo, int N, int H, float scale) {
+                     __nv_bfloat16* __restrict__ out, int64_t ldo, int N, int H, float scale, float* __restrict__ probs) {
   constexpr int kC = HD / 8;             // 16-byte chunks per row
   constexpr int kG = kMapThreads / kC;   // key groups of the P·V pass
   extern __shared__ __align__(16) uint8_t smem_raw[];
@@ -73,6 +74,9 @@ map_attention_kernel(const __nv_bfloat16* __restrict__ kv, int64_t ldkv, const f
   float gsum = 0.f;
 #pragma unroll
   for (int i = 0; i < kMapThreads / 32; ++i) gsum += red[i];
+  if constexpr (kProbs) {
+    for (int n = threadIdx.x; n < N; n += kMapThreads) probs[((int64_t)b * H + h) * N + n] = sc[n] / gsum;
+  }
 
   // out[d] = sum_n p[n] v[n,d] / gsum
   const int g = threadIdx.x / kC, c = threadIdx.x - g * kC;
@@ -101,7 +105,7 @@ map_attention_kernel(const __nv_bfloat16* __restrict__ kv, int64_t ldkv, const f
 
 }  // namespace
 int map_attention_bf16(const void* kv, int64_t ldkv, const float* q, void* out, int64_t ldo, int B, int N,
-                       int H, int hd, float scale, cudaStream_t st) {
+                       int H, int hd, float scale, float* probs, cudaStream_t st) {
   DFD_REQUIRE(kv && q && out, DFD_ERR_BAD_ARG, "map_attention: null pointer");
   DFD_REQUIRE(B > 0 && N > 0 && H > 0, DFD_ERR_SHAPE, "map_attention: B, N, H must be positive");
   DFD_REQUIRE(hd == 64 || hd == 72, DFD_ERR_UNSUPPORTED, "map_attention: head dim %d not supported (64, 72)", hd);
@@ -115,16 +119,20 @@ int map_attention_bf16(const void* kv, int64_t ldkv, const float* q, void* out, 
   DFD_REQUIRE(smem64 <= 200 * 1024, DFD_ERR_UNSUPPORTED, "map_attention: N=%d too long", N);
   const int smem = (int)smem64;
   dim3 grid(H, B);
-  static SmemOptIn smem_once[2];
+  static SmemOptIn smem_once[4];
+  const __nv_bfloat16* k = reinterpret_cast<const __nv_bfloat16*>(kv);
+  __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
+#define DFD_MAP_LAUNCH(HD_, PROBS_, SLOT_)                                                                          \
+  do {                                                                                                              \
+    if (int rc = ensure_dynamic_smem(smem_once[SLOT_], map_attention_kernel<HD_, PROBS_>, 200 * 1024)) return rc;   \
+    map_attention_kernel<HD_, PROBS_><<<grid, kMapThreads, smem, st>>>(k, ldkv, q, o, ldo, N, H, scale, probs);     \
+  } while (0)
   if (hd == 64) {
-    if (int rc = ensure_dynamic_smem(smem_once[0], map_attention_kernel<64>, 200 * 1024)) return rc;
-    map_attention_kernel<64><<<grid, kMapThreads, smem, st>>>(reinterpret_cast<const __nv_bfloat16*>(kv), ldkv, q,
-                                                             reinterpret_cast<__nv_bfloat16*>(out), ldo, N, H, scale);
+    if (probs) DFD_MAP_LAUNCH(64, true, 2); else DFD_MAP_LAUNCH(64, false, 0);
   } else {
-    if (int rc = ensure_dynamic_smem(smem_once[1], map_attention_kernel<72>, 200 * 1024)) return rc;
-    map_attention_kernel<72><<<grid, kMapThreads, smem, st>>>(reinterpret_cast<const __nv_bfloat16*>(kv), ldkv, q,
-                                                             reinterpret_cast<__nv_bfloat16*>(out), ldo, N, H, scale);
+    if (probs) DFD_MAP_LAUNCH(72, true, 3); else DFD_MAP_LAUNCH(72, false, 1);
   }
+#undef DFD_MAP_LAUNCH
   DFD_LAUNCH_CHECK();
   g_launches.fetch_add(1, std::memory_order_relaxed);
   return DFD_OK;
@@ -135,6 +143,6 @@ int map_attention_bf16(const void* kv, int64_t ldkv, const float* q, void* out, 
 extern "C" DFD_API int dfd_map_attention_bf16(const void* kv, int64_t ldkv, const float* q, void* out,
                                               int64_t ldo, int B, int N, int H, int hd, float scale,
                                               void* stream) {
-  return dfd::map_attention_bf16(kv, ldkv, q, out, ldo, B, N, H, hd, scale,
+  return dfd::map_attention_bf16(kv, ldkv, q, out, ldo, B, N, H, hd, scale, nullptr,
                                  reinterpret_cast<cudaStream_t>(stream));
 }

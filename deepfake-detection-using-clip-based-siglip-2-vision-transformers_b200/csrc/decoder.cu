@@ -75,20 +75,6 @@ seg_head_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, const float* _
   if (lane == 0) low[tok] = acc + bias;
 }
 
-// F.interpolate(mode="bilinear", align_corners=False): src = (dst + 0.5) * in/out - 0.5, clamped at 0
-__global__ void __launch_bounds__(256)
-upsample_kernel(const float* __restrict__ low, float* __restrict__ out, int H, int W, int S, float sy, float sx) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, b = blockIdx.z;
-  if (x >= S) return;
-  const float fy = fmaxf((y + 0.5f) * sy - 0.5f, 0.f), fx = fmaxf((x + 0.5f) * sx - 0.5f, 0.f);
-  const int y0 = (int)fy, x0 = (int)fx;
-  const int y1 = min(y0 + 1, H - 1), x1 = min(x0 + 1, W - 1);
-  const float ly = fy - y0, lx = fx - x0;
-  const float* img = low + (int64_t)b * H * W;
-  const float v00 = img[y0 * W + x0], v01 = img[y0 * W + x1], v10 = img[y1 * W + x0], v11 = img[y1 * W + x1];
-  out[((int64_t)b * S + y) * S + x] = (1.f - ly) * ((1.f - lx) * v00 + lx * v01) + ly * ((1.f - lx) * v10 + lx * v11);
-}
-
 // one warp per (row, output): out[b][n] = bias[n] + sum_k x[b][k] * w[n][k]
 __global__ void __launch_bounds__(256)
 linear_small_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, const float* __restrict__ w,
@@ -103,7 +89,32 @@ linear_small_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, const floa
   if (lane == 0) out[o] = acc + (bias ? __ldg(bias + n) : 0.f);
 }
 
+// F.interpolate(mode="bilinear", align_corners=False) of gain·low: src = (dst + 0.5) * in/out - 0.5, clamped at 0
+__global__ void __launch_bounds__(256)
+upsample_kernel(const float* __restrict__ low, float gain, float* __restrict__ out, int H, int W, int S, float sy, float sx) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, b = blockIdx.z;
+  if (x >= S) return;
+  const float fy = fmaxf((y + 0.5f) * sy - 0.5f, 0.f), fx = fmaxf((x + 0.5f) * sx - 0.5f, 0.f);
+  const int y0 = (int)fy, x0 = (int)fx;
+  const int y1 = min(y0 + 1, H - 1), x1 = min(x0 + 1, W - 1);
+  const float ly = fy - y0, lx = fx - x0;
+  const float* img = low + (int64_t)b * H * W;
+  const float v00 = gain * img[y0 * W + x0], v01 = gain * img[y0 * W + x1], v10 = gain * img[y1 * W + x0],
+              v11 = gain * img[y1 * W + x1];
+  out[((int64_t)b * S + y) * S + x] = (1.f - ly) * ((1.f - lx) * v00 + lx * v01) + ly * ((1.f - lx) * v10 + lx * v11);
+}
+
 }  // namespace
+
+// the segmentation head's resize and the attention-rollout heatmap (attention_probs.cu)
+int upsample_bilinear(const float* low, float gain, float* out, int B, int H, int W, int S, cudaStream_t st) {
+  upsample_kernel<<<dim3((S + 255) / 256, S, B), 256, 0, st>>>(low, gain, out, H, W, S, (float)H / (float)S,
+                                                              (float)W / (float)S);
+  DFD_LAUNCH_CHECK();
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  return DFD_OK;
+}
+
 }  // namespace dfd
 
 extern "C" DFD_API int dfd_dwconv3x3_bf16(const void* x, int64_t ldx, const float* w9, const float* bias, void* out,
@@ -134,11 +145,8 @@ extern "C" DFD_API int dfd_seg_head_upsample(const void* x, int64_t ldx, const f
   seg_head_kernel<<<(unsigned)((tokens + 7) / 8), 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), ldx, w, bias,
                                                                 low_scratch, tokens, E);
   DFD_LAUNCH_CHECK();
-  upsample_kernel<<<dim3((S + 255) / 256, S, B), 256, 0, st>>>(low_scratch, out, H, W, S, (float)H / (float)S,
-                                                              (float)W / (float)S);
-  DFD_LAUNCH_CHECK();
-  g_launches.fetch_add(2, std::memory_order_relaxed);
-  return DFD_OK;
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  return upsample_bilinear(low_scratch, 1.0f, out, B, H, W, S, st);
 }
 
 extern "C" DFD_API int dfd_linear_small(const void* x, int64_t ldx, const float* w, const float* bias, float* out, int B,

@@ -81,8 +81,13 @@ int attention_auto_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, 
                         float scale, cudaStream_t st);
 int attention_ws_bf16(const void* qkv, int64_t ldqkv, void* out, int64_t ldo, int B, int N, int H, int hd,
                       float scale, cudaStream_t st);
+// probs != NULL: also writes the probe attention probs[b, h, n] (fp32 [B, H, N])
 int map_attention_bf16(const void* kv, int64_t ldkv, const float* q, void* out, int64_t ldo, int B, int N,
-                       int H, int hd, float scale, cudaStream_t st);
+                       int H, int hd, float scale, float* probs, cudaStream_t st);
+int attention_probs(const void* qkv, int64_t ldqkv, int B, int N, int H, int hd, float scale, int per_head, float* out,
+                    cudaStream_t st);
+// out[b, S, S] = bilinear (align_corners=False) resize of gain·low[b, H, W]
+int upsample_bilinear(const float* low, float gain, float* out, int B, int H, int W, int S, cudaStream_t st);
 
 // ---------------------------------------------------------------------------------------------
 // device helpers

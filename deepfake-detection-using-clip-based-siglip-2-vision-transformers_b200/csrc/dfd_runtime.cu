@@ -27,7 +27,7 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line) {
 }  // namespace dfd
 
 extern "C" DFD_API const char* dfd_last_error(void) { return dfd::t_err; }
-extern "C" DFD_API int dfd_version(void) { return 101; }
+extern "C" DFD_API int dfd_version(void) { return 102; }
 extern "C" DFD_API int64_t dfd_launch_count(void) {
   return dfd::g_launches.load(std::memory_order_relaxed);
 }

@@ -113,6 +113,9 @@ struct dfd_engine {
   float *stats_a, *stats_b;  // per-row (sum, sum of squares) of the residual stream (fuse_ln)
   bool folded;
   void* hidden_tap;          // optional [L+1, B, N, D] bf16 destination of the per-layer hidden states
+  float* attn_tap;           // optional [L, B, (H,) N, N] fp32 destination of the per-layer attention probabilities
+  int attn_per_head;         // 1: [L, B, H, N, N]; 0: head mean [L, B, N, N]
+  float* map_tap;            // optional [B, H, N] fp32 destination of the MAP probe attention
   void* staging;
   int64_t staging_bytes;
   // optional per-launch CUDA-event timing of the forward (bench.py roofline): family 0 GEMM, 1 attention,
@@ -352,6 +355,9 @@ extern "C" DFD_API int dfd_engine_create(const dfd_config* cfg, int device, int 
   e->finalized = false;
   e->folded = false;
   e->hidden_tap = nullptr;
+  e->attn_tap = nullptr;
+  e->attn_per_head = 0;
+  e->map_tap = nullptr;
   e->wslab = e->aslab = nullptr;
   e->staging = nullptr;
   e->staging_bytes = 0;
@@ -493,6 +499,20 @@ extern "C" DFD_API int dfd_engine_set_hidden_tap(dfd_engine* e, void* buf) {
   return DFD_OK;
 }
 
+// attention-map tap (HF output_attentions=True): when attn is set, the next forwards write each layer's attention
+// probabilities right after that layer's attention launch, while its qkv is still live; when map_p is set, the MAP
+// kernel also writes the probe attention.  Not profiled, and the forward runs eagerly while either is set.
+extern "C" DFD_API int dfd_engine_set_attention_tap(dfd_engine* e, float* attn, int per_head, float* map_p) {
+  DFD_REQUIRE(e, DFD_ERR_BAD_ARG, "set_attention_tap: null engine");
+  DFD_REQUIRE(per_head == 0 || per_head == 1, DFD_ERR_BAD_ARG, "set_attention_tap: per_head must be 0 or 1");
+  DFD_REQUIRE(((uintptr_t)attn % 4 == 0) && ((uintptr_t)map_p % 4 == 0), DFD_ERR_BAD_ARG,
+              "set_attention_tap: buffers must be 4-byte aligned");
+  e->attn_tap = attn;
+  e->attn_per_head = per_head;
+  e->map_tap = map_p;
+  return DFD_OK;
+}
+
 extern "C" DFD_API int dfd_engine_profile(dfd_engine* e, int enable) {
   DFD_REQUIRE(e, DFD_ERR_BAD_ARG, "profile: null engine");
   DeviceGuard guard(e->device);
@@ -578,6 +598,9 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
       DFD_OP(5, gemm_bf16_dispatch(e->h, D, l.w_qkv, D, e->qkv, 3 * D, M, 3 * D, D, &ep, 0, st));
     }
     DFD_OP(1, attention_auto_bf16(e->qkv, 3 * D, e->att, D, B, N, H, hd, scale, st));
+    if (e->attn_tap)
+      DFD_TRY(attention_probs(e->qkv, 3 * D, B, N, H, hd, scale, e->attn_per_head,
+                              e->attn_tap + (int64_t)li * B * (e->attn_per_head ? H : 1) * N * N, st));
     {
       dfd_gemm_epilogue ep{};
       ep.bias = l.b_o;
@@ -624,7 +647,7 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
     ep.bias = e->b_in + D;
     DFD_OP(0, gemm_bf16_dispatch(xp, D, e->w_in + (int64_t)D * D, D, e->qkv, 2 * D, M, 2 * D, D, &ep, 0, st));
   }
-  DFD_OP(4, map_attention_bf16(e->qkv, 2 * D, e->q_probe, e->ao, D, B, N, H, hd, scale, st));
+  DFD_OP(4, map_attention_bf16(e->qkv, 2 * D, e->q_probe, e->ao, D, B, N, H, hd, scale, e->map_tap, st));
   {
     dfd_gemm_epilogue ep{};
     ep.bias = e->b_mo;
@@ -652,7 +675,8 @@ static int forward_body(dfd_engine* e, const void* pixels, int pix_format, int B
 // device.  With graphs on, a call signature (pointers, batch, input geometry) runs eagerly the first time it is seen, is
 // captured the second time (on a private stream: the caller's may be the legacy default stream, which cannot capture) and
 // is replayed with ONE cudaGraphLaunch on the caller's stream from then on: tensor maps and kernel arguments are baked into
-// the graph.  Up to kMaxGraphs signatures are kept (least recently used out).  Profiling and hidden-state taps run eagerly.
+// the graph.  Up to kMaxGraphs signatures are kept (least recently used out).  Profiling, hidden-state and attention taps
+// run eagerly.
 extern "C" DFD_API int dfd_engine_set_graphs(dfd_engine* e, int enable) {
   DFD_REQUIRE(e, DFD_ERR_BAD_ARG, "set_graphs: null engine");
   e->graphs_on = enable != 0;
@@ -706,7 +730,8 @@ extern "C" DFD_API int dfd_engine_forward(dfd_engine* e, const void* pixels, int
                 e->device, cur);
   }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const bool eager = !e->graphs_on || e->prof_on || e->hidden_tap != nullptr;
+  const bool eager =
+      !e->graphs_on || e->prof_on || e->hidden_tap != nullptr || e->attn_tap != nullptr || e->map_tap != nullptr;
   if (eager) return forward_body(e, pixels, pix_format, B, Hin, Win, resize_mode, pooled, last_hidden, st);
 
   constexpr size_t kMaxGraphs = 16;

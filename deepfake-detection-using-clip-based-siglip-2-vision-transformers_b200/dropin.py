@@ -694,7 +694,8 @@ def interpolated_position_table(pos: torch.Tensor, new_grid: int) -> torch.Tenso
 class SiglipVisionModel:
     """HF-shaped wrapper: `SiglipVisionModel.from_state_dict(sd)(pixel_values=x)` -> .pooler_output [B,D] f32,
     .last_hidden_state [B,N,D], and with output_hidden_states=True the tuple of L+1 per-layer states
-    (Siglip2sidafrozen.py:753,787-793).  `interpolate_pos_encoding=True` (Siglip2sidafrozen.py:787, progressive resize
+    (Siglip2sidafrozen.py:753,787-793).  output_attentions=True adds .attentions, the tuple of L fp32 [B,H,N,N]
+    attention probabilities that HF returns under eager attention (None otherwise).  `interpolate_pos_encoding=True` (Siglip2sidafrozen.py:787, progressive resize
     :975-987) accepts other square resolutions: each new patch grid gets its own engine (workspace sized for that token
     count) whose position table is the bicubic resample of the trained one."""
 
@@ -734,7 +735,7 @@ class SiglipVisionModel:
         return self._engines[grid]
 
     def __call__(self, pixel_values: torch.Tensor, output_hidden_states: bool = False,
-                 interpolate_pos_encoding: bool = False, **_):
+                 interpolate_pos_encoding: bool = False, output_attentions: bool = False, **_):
         P = self.arch.patch_size
         H, W = pixel_values.shape[-2:]
         gh, gw = H // P, W // P
@@ -749,15 +750,25 @@ class SiglipVisionModel:
             raise NotImplementedError("interpolate_pos_encoding for non-square inputs is not built (the reference's "
                                       "SigLIP2_MTL needs square token grids too: Siglip2sidafrozen.py:795-801)")
         x = pixel_values.to(self.device).float()
+        if output_attentions:  # HF eager: a tuple of L fp32 [B,H,N,N]; one engine forward per chunk gives every output
+            chunks = [eng._forward_tapped(x[i:i + eng.max_batch], 0, True, output_hidden_states, True)
+                      for i in range(0, x.shape[0], eng.max_batch)]
+            pooled = torch.cat([c[0] for c in chunks])
+            last = torch.cat([c[1] for c in chunks])
+            attn = torch.cat([c[2] for c in chunks], 1)
+            hid = tuple(h.float() for h in torch.cat([c[4] for c in chunks], 1)) if output_hidden_states else None
+            return types.SimpleNamespace(pooler_output=pooled.float(), last_hidden_state=last.float(), hidden_states=hid,
+                                         attentions=tuple(attn.unbind(0)))
         if output_hidden_states:  # tuple of L+1 tensors, as SigLIP2_MTL consumes them (Siglip2sidafrozen.py:790-793)
             chunks = [eng.forward_hidden(x[i:i + eng.max_batch]) for i in range(0, x.shape[0], eng.max_batch)]
             pooled = torch.cat([c[0] for c in chunks])
             last = torch.cat([c[1] for c in chunks])
             hid = torch.cat([c[2] for c in chunks], 1)
             return types.SimpleNamespace(pooler_output=pooled.float(), last_hidden_state=last.float(),
-                                         hidden_states=tuple(h.float() for h in hid))
+                                         hidden_states=tuple(h.float() for h in hid), attentions=None)
         pooled, last = eng(x, want_last_hidden=True)
-        return types.SimpleNamespace(pooler_output=pooled.float(), last_hidden_state=last.float(), hidden_states=None)
+        return types.SimpleNamespace(pooler_output=pooled.float(), last_hidden_state=last.float(), hidden_states=None,
+                                     attentions=None)
 
 
 def install_import_shims() -> None:

@@ -238,6 +238,34 @@ class SiglipEngine:
             check(self._lib.dfd_engine_set_hidden_tap(self._h, None))
         return pooled, last, hidden
 
+    def forward_attentions(self, pixels: torch.Tensor, resize_mode: int = 0, per_head: bool = False,
+                           hidden: bool = False):
+        """One forward that also returns the attention maps (HF `output_attentions=True`): (pooled [B,D] bf16,
+        attentions fp32 [L,B,N,N] (head mean) or [L,B,H,N,N] (per_head), map_attention fp32 [B,H,N] = the MAP probe's
+        attention over the tokens[, hidden [L+1,B,N,D] bf16 with hidden=True]).  Rows sum to 1.  B <= max_batch."""
+        pooled, _, attn, map_p, hid = self._forward_tapped(pixels, resize_mode, per_head, hidden, False)
+        return (pooled, attn, map_p, hid) if hidden else (pooled, attn, map_p)
+
+    def _forward_tapped(self, pixels, resize_mode, per_head, hidden, want_last_hidden):
+        B = pixels.shape[0]
+        if B > self.max_batch:
+            raise ValueError("forward_attentions: batch must fit the engine workspace (max_batch)")
+        a = self.arch
+        L, H, N = a.num_hidden_layers, a.num_attention_heads, a.tokens
+        shape = (L, B, H, N, N) if per_head else (L, B, N, N)
+        attn = torch.empty(shape, dtype=torch.float32, device=self.device)
+        map_p = torch.empty((B, H, N), dtype=torch.float32, device=self.device)
+        hid = (torch.empty((L + 1, B, N, a.hidden_size), dtype=torch.bfloat16, device=self.device) if hidden else None)
+        check(self._lib.dfd_engine_set_attention_tap(self._h, attn.data_ptr(), int(bool(per_head)), map_p.data_ptr()))
+        try:
+            if hid is not None:
+                check(self._lib.dfd_engine_set_hidden_tap(self._h, hid.data_ptr()))
+            pooled, last = self.forward(pixels, resize_mode, want_last_hidden=want_last_hidden)
+        finally:
+            check(self._lib.dfd_engine_set_attention_tap(self._h, None, 0, None))
+            check(self._lib.dfd_engine_set_hidden_tap(self._h, None))
+        return pooled, last, attn, map_p, hid
+
     def forward(self, pixels: torch.Tensor, resize_mode: int = 0, want_last_hidden: bool = False):
         """pixels: uint8 [B,H,W,3] or float32 [B,3,H,W] on this engine's device.  Batches larger than
         max_batch are processed in chunks.  Returns (pooled bf16 [B,D], last_hidden bf16 [B,N,D] | None)."""

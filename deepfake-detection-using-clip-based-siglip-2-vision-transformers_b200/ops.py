@@ -140,6 +140,38 @@ def attention_bf16(qkv: torch.Tensor, B: int, N: int, H: int, hd: int, scale: Op
     return out
 
 
+def attention_probs(qkv: torch.Tensor, B: int, N: int, H: int, hd: int, scale: Optional[float] = None,
+                    per_head: bool = True) -> torch.Tensor:
+    """The attention probabilities softmax(q k^T scale) of the packed qkv that attention_bf16 reads, in fp32:
+    [B, H, N, N] with per_head, else the head mean [B, N, N]."""
+    _need_cuda(qkv)
+    assert qkv.dtype == torch.bfloat16 and qkv.dim() == 2 and qkv.shape[0] == B * N and qkv.stride(1) == 1
+    shape = (B, H, N, N) if per_head else (B, N, N)
+    out = torch.empty(shape, dtype=torch.float32, device=qkv.device)
+    scale = (1.0 / math.sqrt(hd)) if scale is None else scale
+    check(_lib.load().dfd_attention_probs(qkv.data_ptr(), qkv.stride(0), B, N, H, hd, scale, int(bool(per_head)),
+                                          out.data_ptr(), current_stream()))
+    return out
+
+
+def attention_rollout(attn_mean: torch.Tensor, map_p: torch.Tensor, alpha: float = 0.5, heatmap_size: int = 0):
+    """Attention rollout seeded by the MAP probe: attn_mean fp32 [L, B, N, N] (head-mean probabilities per layer),
+    map_p fp32 [B, H, N].  Returns (relevance [B, N], heatmap [B, S, S] | None).  The heatmap (heatmap_size = S > 0,
+    needs a square token grid) is the bilinear upsample of N·relevance, so 1.0 marks a uniform share."""
+    _need_cuda(attn_mean, map_p)
+    assert attn_mean.dtype == torch.float32 and attn_mean.dim() == 4 and attn_mean.is_contiguous()
+    assert map_p.dtype == torch.float32 and map_p.dim() == 3 and map_p.is_contiguous()
+    L, B, N, _ = attn_mean.shape
+    H = map_p.shape[1]
+    assert attn_mean.shape == (L, B, N, N) and map_p.shape == (B, H, N)
+    rel = torch.empty((B, N), dtype=torch.float32, device=map_p.device)
+    heat = (torch.empty((B, heatmap_size, heatmap_size), dtype=torch.float32, device=map_p.device)
+            if heatmap_size > 0 else None)
+    check(_lib.load().dfd_attention_rollout(attn_mean.data_ptr(), map_p.data_ptr(), L, B, N, H, float(alpha),
+                                            math.isqrt(N), heatmap_size, rel.data_ptr(), _p(heat), current_stream()))
+    return rel, heat
+
+
 def map_attention_bf16(kv: torch.Tensor, q: torch.Tensor, B: int, N: int, H: int, hd: int,
                        scale: Optional[float] = None) -> torch.Tensor:
     _need_cuda(kv, q)

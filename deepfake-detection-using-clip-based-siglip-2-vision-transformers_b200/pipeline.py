@@ -134,6 +134,26 @@ class DetectionPipeline:
         out["pooled"] = pooled
         return out
 
+    @_on_own_device
+    def explain(self, images_u8: torch.Tensor, resize_mode: int = 0, alpha: float = 0.5) -> Dict[str, torch.Tensor]:
+        """Where the backbone looks: attention rollout (Abnar & Zuidema 2020) seeded by the MAP pooling probe, the query
+        that forms the pooled embedding.  images_u8: u8 NHWC on the device.  Returns {"relevance" [B,G,G] (sums to 1 per
+        image), "heatmap" [B,S,S] (bilinear upsample of G²·relevance: 1.0 = a uniform share, above 1 = more than its
+        share), "z_sig" [B] (the classifier logit of the same forward)}.  The maps are not normalised; to display one,
+        scale it to [0, 1] per image (or clip at a fixed multiple of the uniform share) and overlay it on the image.
+        Runs in chunks of at most max_batch images; the head-mean probabilities take L·N²·4 bytes per image."""
+        a, eng = self.arch, self.engine
+        G, S = a.grid, a.image_size
+        rel, heat, z = [], [], []
+        for i in range(0, images_u8.shape[0], eng.max_batch):
+            pooled, attn, map_p = eng.forward_attentions(images_u8[i:i + eng.max_batch], resize_mode)
+            r, h = ops.attention_rollout(attn, map_p, alpha, S)
+            del attn
+            rel.append(r.view(-1, G, G))
+            heat.append(h)
+            z.append(ops.head_fwd(self.head, pooled)[1])
+        return {"relevance": torch.cat(rel), "heatmap": torch.cat(heat), "z_sig": torch.cat(z)}
+
     @staticmethod
     def pack(out: Dict[str, torch.Tensor]) -> torch.Tensor:
         """[B, 14] fp32 score records (PACKED_FIELDS) — the unit that is all-gathered across ranks."""

@@ -148,6 +148,23 @@ DFD_API int dfd_map_attention_bf16(const void* kv, int64_t ldkv, const float* q,
                                    int64_t ldo, int B, int N, int H, int hd, float scale,
                                    void* stream);
 
+/* Attention probabilities of the packed qkv that dfd_attention_bf16 reads (same layout, hd in {64,72}, any N >= 1):
+ * P = softmax(q·kᵀ·scale) in fp32 (HF eager_attention_forward's attn_weights, HF:modeling_siglip.py:229-249), scale > 0.
+ *   per_head = 1: out [B, H, N, N]  (what HF output_attentions returns)
+ *   per_head = 0: out [B, N, N] = (1/H)·Σ_h P_h, summed on chip (the input of the rollout below)
+ * S = q·kᵀ runs on the tensor cores; two sweeps over the keys (row statistics, then the probabilities). */
+DFD_API int dfd_attention_probs(const void* qkv, int64_t ldqkv, int B, int N, int H, int hd, float scale, int per_head,
+                                float* out, void* stream);
+
+/* Attention rollout (Abnar & Zuidema 2020) seeded by the MAP probe, which is the query that forms the pooled embedding
+ * (SigLIP has no CLS token): r = mean_h map_p[b, h, :], then for l = L-1 ... 0: r <- alpha·(r·attn_mean[l][b]) +
+ * (1 - alpha)·r.  relevance [B][N] sums to 1.  heatmap (optional, needs G·G == N) [B][S][S] = the bilinear
+ * (align_corners=False) resize of N·relevance on the G×G grid, so 1.0 is a uniform share.  Uses B·N floats of
+ * stream-ordered scratch. */
+DFD_API int dfd_attention_rollout(const float* attn_mean /*[L][B][N][N]*/, const float* map_p /*[B][H][N]*/, int L, int B,
+                                  int N, int H, float alpha, int G, int S, float* relevance /*[B][N]*/,
+                                  float* heatmap /*[B][S][S] or NULL*/, void* stream);
+
 /* Classifier head on pooled embeddings (fp32 weights, fp32 math):
  *   f = pooled / (‖pooled‖₂ + norm_eps)                       inference_ai_human_images.py:149; +1e-6: train_fusion_head_only.py:106
  *   then, if kind >= 1: [kind 2: SE gate f·sigmoid(W2·relu(W1·f))  train_fusion_head_only.py:84-89,107]
@@ -329,6 +346,12 @@ DFD_API int dfd_engine_forward(dfd_engine* e, const void* pixels, int pix_format
  * forwards also copy the embedding output and each encoder layer's output to buf as bf16 [L+1][B][N][D] (B = the
  * batch of that forward).  NULL switches the tap off. */
 DFD_API int dfd_engine_set_hidden_tap(dfd_engine* e, void* buf);
+/* Attention maps (HF output_attentions=True): when attn != NULL the following forwards write layer l's attention
+ * probabilities to attn + l·(per-layer size), in the layout of dfd_attention_probs(per_head): fp32 [L][B][H][N][N]
+ * (per_head = 1) or the head mean [L][B][N][N] (per_head = 0).  When map_p != NULL the MAP pooling kernel also writes the
+ * probe attention, fp32 [B][H][N].  NULL / NULL switches the tap off.  While it is on, forwards run eagerly (no graph
+ * replay); its launches are not profiled. */
+DFD_API int dfd_engine_set_attention_tap(dfd_engine* e, float* attn, int per_head, float* map_p);
 /* CUDA graphs of the forward: with enable != 0 a call signature (pixels / pooled / last_hidden pointers, batch, input geometry)
  * runs eagerly the first time, is captured the second time and replayed with one cudaGraphLaunch on the caller's stream
  * afterwards (tensor maps and arguments baked in; 16 signatures kept, LRU).  Keep the buffers of a serving loop stable to
