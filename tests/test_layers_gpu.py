@@ -85,12 +85,13 @@ def _cell_rms(e):
     return (s / (rows[:, None] * COL_CHUNK)).sqrt()
 
 
-def _gate_ratios(out, ref, emu):
-    """(ALPHA, KAPPA, BETA) that the engine's output `out` needs: the smallest values with which it passes the gates."""
+def _gate_ratios(out, ref, emu, stored=torch.bfloat16):
+    """(ALPHA, KAPPA, BETA) that the engine's output `out` needs: the smallest values with which it passes the gates.
+    The emulation is rounded to `stored`, the dtype in which the engine stores the output."""
     if out.dim() == 2:   # pooled [B, D]: one row per image
         out, ref, emu = out[:, None], ref[:, None], emu[:, None]
     e = out.double() - ref
-    e_emu = emu.to(torch.bfloat16).double() - ref
+    e_emu = emu.to(stored).double() - ref
     rms_emu = e_emu.square().mean().sqrt()
     alpha = e.square().mean().sqrt() / rms_emu
     kappa = (_cell_rms(e) / _cell_rms(e_emu)).max()
